@@ -2,7 +2,7 @@
 """bench.py -- lag-evaluations/s of the helioprojective pointing search on BASELINE.json configs[0]
 (HRIEUV-like 2048^2 vs FSI-174-like 3072^2, 60x60 CRVAL lags at 1 arcsec, synthetic FITS).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over the whole 3600-lag grid (homographies + fused lag kernel + finalize, plus
 the all-gather of the cube when N > 1; the lag list is sharded over the N ranks => strong scaling). The headline is
@@ -25,6 +25,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -92,7 +93,9 @@ def measured_constants():
 
 
 def synth_dir():
-    d = os.environ.get("COREG_BENCH_DATA", "/tmp/coreg_bench_data")
+    """Cache of the seeded synthetic inputs (outside the source tree, which may be read-only). Per user: in a shared
+    temporary directory another user's copy is not writable."""
+    d = os.environ.get("COREG_BENCH_DATA") or os.path.join(tempfile.gettempdir(), f"coreg_bench_data_{os.getuid()}")
     os.makedirs(d, exist_ok=True)
     return d
 
@@ -632,6 +635,9 @@ def run_gpu(args):
         ms_total = timed_device(ctx, step, args.steps, 0)
         k_ms, k_n = _ext.profile_end()
         flagged = eng.resolve_flags(tab_dev, local_out[:hi - lo])   # mixed only
+        if world > 1:
+            dist.all_gather_into_tensor(full, local_out)
+        last = (full[:n_lags] if world > 1 else local_out[:n_lags]).cpu().numpy()   # the last timed step's cube
         # evaluated (pixel, lag) pairs of this rank's slice: what the roofline counts (one more pass, untimed)
         nv = torch.zeros(max(hi - lo, 1), dtype=torch.int64, device=eng.device)
         if hi > lo:
@@ -640,8 +646,8 @@ def run_gpu(args):
         if world > 1:
             dist.all_gather_into_tensor(full, local_out)
         cube = (full[:n_lags] if world > 1 else local_out[:n_lags]).cpu().numpy()
-        return dict(ms=ms_total / args.steps, k_ms=k_ms / max(1, k_n), k_n=k_n, cube=cube, eng=eng, table=table,
-                    lo=lo, hi=hi, n_lags=n_lags, flagged=int(ctx.sum_over_ranks(flagged)),
+        return dict(ms=ms_total / args.steps, k_ms=k_ms / max(1, k_n), k_n=k_n, cube=cube, last=last, eng=eng,
+                    table=table, lo=lo, hi=hi, n_lags=n_lags, flagged=int(ctx.sum_over_ranks(flagged)),
                     evaluated=float(nv[:hi - lo].sum().item()) if hi > lo else 0.0,
                     fast=table.shape[1] == _ext.TAN_WCS_DOUBLES)
 
@@ -650,6 +656,10 @@ def run_gpu(args):
         sampler.start()
     main = device_arm(args.arithmetic or "fp64")
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # what a caller of the timed path receives: r per lag, flat in the lag order of the cube (lag_crval1 major)
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "corr.npy"), main["last"].astype(np.float64))
     eng, table, n_lags, lo, hi = main["eng"], main["table"], main["n_lags"], main["lo"], main["hi"]
     value = n_lags / (main["ms"] * 1e-3)
     mixed = None
@@ -667,7 +677,7 @@ def run_gpu(args):
     # host inputs: the images as the FITS files hold them (float32), in pinned memory
     h_large = torch.from_numpy(np.ascontiguousarray(a.data_large)).pin_memory().numpy()
     h_small = torch.from_numpy(np.ascontiguousarray(a.data_small)).pin_memory().numpy()
-    e2e_steps = max(1, min(args.steps, 5))
+    e2e_steps = args.steps
 
     def e2e_step():
         e = E.LagSearchEngine(order=2, strict=args.strict, variant=args.variant, small_storage=args.small_storage,
@@ -706,7 +716,7 @@ def run_gpu(args):
     configs = {}
     if not args.no_secondary:
         for name, fn in (("configs1_carrington",
-                          lambda: carrington_secondary(pl, ps, max(3, min(args.steps, 10)), world, barrier, torch, dist,
+                          lambda: carrington_secondary(pl, ps, args.steps, world, barrier, torch, dist,
                                                        args.carrington_variant, fp64_peak=fp64_peak)),
                          ("configs2_spice", lambda: spice_secondary(ctx, rank)),
                          ("configs3_grid5d", lambda: grid5d_secondary(ctx, pl, ps)),
@@ -833,8 +843,10 @@ def run_gpu(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed loop (headline, e2e, configs[1])")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the headline cube of the last step to DIR/corr.npy (float64)")
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--strict", action="store_true", help="scipy operation order in the spline (no FMA)")
     ap.add_argument("--variant", type=int, default=0, help="kernel tuning variant (rows per thread / occupancy)")
@@ -850,7 +862,11 @@ def main():
     ap.add_argument("--frames", type=int, default=SEQUENCE_FRAMES, help="frame searches of configs[4]")
     ap.add_argument("--carrington-variant", type=int, default=0)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs writes the GPU arm's cube; the reference arm times a sample of lags")
         return run_reference(args)
     return run_gpu(args)
 

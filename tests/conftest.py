@@ -40,6 +40,14 @@ def toy_rect_pair(tmp_path_factory):
     return p_large, p_small, spec
 
 
+@pytest.fixture(scope="session")
+def config1_pair(tmp_path_factory):
+    """BASELINE configs[0] pair (2048^2 small vs 3072^2 large, the scene bench.py times), written once per session."""
+    from euispice_coreg_b200._synth.scene import make_config1
+    p_large, p_small, _ = make_config1(str(tmp_path_factory.mktemp("config1")))
+    return p_large, p_small
+
+
 def load_pair(p_large, p_small):
     from euispice_coreg_b200._compat import fits_lite
     L, S = fits_lite.open(p_large)[0], fits_lite.open(p_small)[0]

@@ -36,9 +36,8 @@ def torch_cuda():
 
 
 @pytest.fixture(scope="module")
-def config1():
-    import bench
-    pl, ps = bench.ensure_config1()
+def config1(config1_pair):
+    pl, ps = config1_pair
     dl, _, ds, _ = load_pair(pl, ps)
     h = hashlib.sha256()
     h.update(np.ascontiguousarray(dl).tobytes())

@@ -323,7 +323,7 @@ def test_hard_images_stay_inside_the_contract(torch_cuda, toy_pair, tmp_path, ki
             assert flagged == 0 and not np.array_equal(gpu, f64) and np.nanmax(np.abs(gpu - f64)) < 1e-7
 
 
-def test_mixed_kernel_on_low_contrast_image_at_full_size(torch_cuda, tmp_path):
+def test_mixed_kernel_on_low_contrast_image_at_full_size(torch_cuda, config1_pair, tmp_path):
     """BASELINE configs[0] with the small image rescaled to mean 3e4, sigma 1 (float32 ulp of a pixel value = 2e-3
     sigma): with 4e6 samples per lag the mixed kernel's error model stays under 1e-7, no lag is flagged, and the whole
     3600-lag cube agrees with the all-FP64 kernel to 1e-7 -- whose own distance to the oracle is checked on a
@@ -332,7 +332,7 @@ def test_mixed_kernel_on_low_contrast_image_at_full_size(torch_cuda, tmp_path):
     import bench
     from euispice_coreg_b200.hdrshift import Alignment
     from oracle.hpc import HpcSearch, cube_multiprocess
-    pair = _rewrite_small(bench.ensure_config1(), tmp_path, "cfg1_low_contrast", HARD_IMAGES["low_contrast"])
+    pair = _rewrite_small(config1_pair, tmp_path, "cfg1_low_contrast", HARD_IMAGES["low_contrast"])
     cubes = {}
     for arith in ("fp64", "mixed"):
         a = Alignment(pair[0], pair[1], parallelism=True, arithmetic=arith, **bench.LAGS)
@@ -461,7 +461,7 @@ _CFG1_REF = {}
 
 
 @ARITH
-def test_config1_full_size_bounded_sample_vs_oracle(torch_cuda, arithmetic):
+def test_config1_full_size_bounded_sample_vs_oracle(torch_cuda, config1_pair, arithmetic):
     """BASELINE.json configs[0] at full size (2048^2 vs 3072^2, 60x60 CRVAL lags): the whole GPU cube through the
     public API against the oracle on a bounded sample of lags (the oracle needs ~5 s per lag per core).
 
@@ -473,7 +473,7 @@ def test_config1_full_size_bounded_sample_vs_oracle(torch_cuda, arithmetic):
     import bench
     from euispice_coreg_b200.hdrshift import Alignment
     from oracle.hpc import HpcSearch, cube_multiprocess
-    pl, ps = bench.ensure_config1()
+    pl, ps = config1_pair
     a = Alignment(pl, ps, parallelism=True, arithmetic=arithmetic, **bench.LAGS)
     cube = a.align_using_helioprojective(return_type="corr")
     assert cube.shape == (60, 60, 1, 1, 1, 1)
@@ -561,7 +561,7 @@ def test_single_lag_and_tiny_images(torch_cuda, tmp_path):
     assert gpu.shape == (1, 1, 1, 1, 1, 1) and abs(gpu.item() - ref.item()) <= R_TOL
 
 
-def test_config1_full_size_properties(torch_cuda):
+def test_config1_full_size_properties(torch_cuda, config1_pair):
     """Size-independent properties at BASELINE's full size (2048^2, 3600 lags), where the oracle is too slow to
     check every lag: (1) the cube does not depend on how the lag list is sliced or ordered (bitwise); (2) Pearson's
     r is invariant under a positive affine map of the small image -- scaling by 2 is exact in binary floating
@@ -570,7 +570,7 @@ def test_config1_full_size_properties(torch_cuda):
     import bench
     from euispice_coreg_b200._compat.wcs import TanWcs
     from euispice_coreg_b200.hdrshift import Alignment, engine
-    pl, ps = bench.ensure_config1()
+    pl, ps = config1_pair
     a = Alignment(pl, ps, parallelism=True, **bench.LAGS)
     cube = a.align_using_helioprojective(return_type="corr").ravel()
     eng = a.engine

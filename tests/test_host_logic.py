@@ -204,7 +204,7 @@ def test_alignment_results_on_reference_golden_cube():
     assert 22.0 < rb.shift_arcsec[0] < 26.0 and 5.0 < rb.shift_arcsec[1] < 9.0
 
 
-def test_alignment_results_quirks_kept():
+def test_alignment_results_quirks_kept(tmp_path):
     """Reference quirks (AlignmentResults.py:224-239): offsets of -2 wrap around below index 0, so a lag axis of
     length 1 raises IndexError exactly like the reference; an all-NaN cube raises ValueError (nanargmax)."""
     from euispice_coreg_b200.hdrshift import AlignmentResults
@@ -219,7 +219,7 @@ def test_alignment_results_quirks_kept():
                          lag_cdelt2=None, lag_crota=None, unit_lag="arcsec")
     assert tuple(int(v) for v in r.max_index[:2]) == (1, 2) and len(r.shift_arcsec) == 5
     with pytest.raises(ValueError):
-        r.write_corrected_fits([0], "/tmp/nowhere.fits")
+        r.write_corrected_fits([0], str(tmp_path / "nowhere.fits"))
     c = np.full((3, 3, 1, 1, 1, 1), np.nan)
     with pytest.raises(ValueError):
         AlignmentResults(corr=c, lag_crval1=[1, 2, 3], lag_crval2=[1, 2, 3], lag_cdelt1=None, lag_cdelt2=None,
@@ -394,9 +394,9 @@ if rank == 0:
 def test_lag_and_frame_sharding_gather_gloo(tmp_path, world):
     script = tmp_path / "gloo_worker.py"
     script.write_text(_GLOO.format(root=ROOT))
-    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={world}",
-                          "--master-addr", "127.0.0.1", "--master-port", str(29531 + world), str(script)],
-                         capture_output=True, text=True, timeout=300)
+    # --standalone: the launcher picks a free local port, so concurrent runs on one host do not collide
+    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", f"--nproc-per-node={world}",
+                          str(script)], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr[-2000:]
     assert "GLOO_OK" in out.stdout
 
