@@ -559,6 +559,14 @@ class Alignment:
         return (float(np.radians(hdr["HGLN_OBS"])), float(np.radians(hdr["HGLT_OBS"])), float(hdr["DSUN_OBS"]),
                 timeutil.to_seconds(date))
 
+    def _surface_frames(self, d_solar_r):
+        """`_ext.CoregSurfaceFrames` of the pair: the small image's observer as target, the large image's as source."""
+        from .. import _ext
+        g_lon, g_lat, g_d, g_t = self._surface_frame(self.hdr_small)
+        i_lon, i_lat, i_d, i_t = self._surface_frame(self.hdr_large)
+        return _ext.CoregSurfaceFrames(g_lon, g_lat, g_d, i_lon, i_lat, i_d, (i_t - g_t) / 86400.0,
+                                       d_solar_r * _engine.R_SUN_M)
+
     def _surface_search(self, eng, refs, d1, d2, d3, d4, d5, d_solar_r):
         """`_carrington_transform_sunpy` (`alignment.py:939-985`) on the device. Once: the large image reprojected onto
         the small image's grid through sunpy's helioprojective -> helioprojective change of observer for points on the
@@ -568,14 +576,9 @@ class Alignment:
         the change of frame is the identity and the call is the helioprojective search's geometry with bilinear
         interpolation and reproject's edge rule, no float32 store. sunpy / reproject are absent from the image: the
         algorithm is restated from its published form (oracle/surface_reproject.py), parity unpinned."""
-        from .. import _ext
         w_small = TanWcs.from_header(self.hdr_small)
         w_large = TanWcs.from_header(self.hdr_large)
-        g_lon, g_lat, g_d, g_t = self._surface_frame(self.hdr_small)
-        i_lon, i_lat, i_d, i_t = self._surface_frame(self.hdr_large)
-        frames = _ext.CoregSurfaceFrames(g_lon, g_lat, g_d, i_lon, i_lat, i_d, (i_t - g_t) / 86400.0,
-                                         d_solar_r * _engine.R_SUN_M)
-        eng.prepare_surface(self.data_large, w_large, w_small, frames)
+        eng.prepare_surface(self.data_large, w_large, w_small, self._surface_frames(d_solar_r))
         self.hdr_large = self.hdr_small.copy()
         table, dead = eng.surface_lag_table(self.hdr_small, refs, d1, d2, d3, d4, d5, self.cdelt_semantics)
         corr, nvalid = eng.search(table, return_nvalid=True)
@@ -586,19 +589,26 @@ class Alignment:
         """Per CROTA-lag value one pair of detector planes; CRVAL lags are pure offsets on them
         (`alignment.py:889-901`, `utils/rectify.py:377-423`)."""
         for hdr in (self.hdr_small, self.hdr_large):
-            if str(hdr["CUNIT1"]).strip() != "arcsec":
-                warnings.warn("the 'fa' Carrington transform assumes arcsec headers (utils/rectify.py:362-363)")
+            warn_fa_units(hdr)
         eng.prepare_carrington_large(self.data_large, self.hdr_large, d_solar_r, self.lonlims, self.latlims,
                                      self.shape)
         n = d1.size
         corr = np.zeros(n, dtype=np.float64)
         nvalid = np.zeros(n, dtype=np.int64)
-        dead = np.zeros(n, dtype=bool)
-        if self.cdelt_semantics == "reference":
-            dead = d4 != 0.0
-        elif (np.any(d3 != 0.0) or np.any(d4 != 0.0)):
-            raise NotImplementedError("CDELT lags in the Carrington frame need cdelt_semantics='reference'")
+        dead = carrington_dead_lags(d3, d4, self.cdelt_semantics)
+        for sel, planes, table, lag_ij in self._carrington_tables(eng, refs, d1, d2, d5, dead, d_solar_r):
+            c, nv = eng.search(table, planes=planes, return_nvalid=True, lag_ij=lag_ij)
+            corr[sel] = c
+            nvalid[sel] = nv
+        return corr, nvalid
+
+    def _carrington_tables(self, eng, refs, d1, d2, d5, dead, d_solar_r):
+        """Per CROTA-lag value (generated one at a time: each holds a pair of planes the size of the grid):
+        (flat indices of its lags, detector planes (tx, ty) of the rotated header on the Carrington grid, [n, 2] (x0, y0)
+        offset table, CRVAL grid indices for `offset_patch_order`). Lags in `dead` are left out."""
         roll_ref = self.hdr_small["CROTA"] if "CROTA" in self.hdr_small else self.hdr_small["CROTA2"]
+        shape5 = (len(self.lag_crval1), len(self.lag_crval2), len(self.lag_cdelt1), len(self.lag_cdelt2),
+                  len(self.lag_crota))
         for dc in np.unique(d5):
             sel = np.nonzero((d5 == dc) & ~dead)[0]
             if sel.size == 0:
@@ -613,10 +623,20 @@ class Alignment:
             table = np.stack([x0, y0], axis=1).astype(np.float64)
             # CRVAL grid indices of the selected lags (flat C order: crval1 slowest ... crota fastest): the kernel
             # takes them in detector-plane patches; lags that differ only in a CDELT index never share a patch
-            shape5 = (len(self.lag_crval1), len(self.lag_crval2), len(self.lag_cdelt1), len(self.lag_cdelt2),
-                      len(self.lag_crota))
             i1, i2, i3, i4, _ = np.unravel_index(sel, shape5)
-            c, nv = eng.search(table, planes=planes, return_nvalid=True, lag_ij=(i1, i2, i3 * shape5[3] + i4))
-            corr[sel] = c
-            nvalid[sel] = nv
-        return corr, nvalid
+            yield sel, planes, table, (i1, i2, i3 * shape5[3] + i4)
+
+
+def warn_fa_units(hdr):
+    if str(hdr["CUNIT1"]).strip() != "arcsec":
+        warnings.warn("the 'fa' Carrington transform assumes arcsec headers (utils/rectify.py:362-363)")
+
+
+def carrington_dead_lags(d_cdelt1, d_cdelt2, cdelt_semantics):
+    """Lags of the 'fa' Carrington search the reference cannot evaluate (a CDELT2 lag: they read 0.0 in the cube);
+    CDELT lags under any other semantics are not implemented in this frame."""
+    if cdelt_semantics == "reference":
+        return np.asarray(d_cdelt2) != 0.0
+    if np.any(np.asarray(d_cdelt1) != 0.0) or np.any(np.asarray(d_cdelt2) != 0.0):
+        raise NotImplementedError("CDELT lags in the Carrington frame need cdelt_semantics='reference'")
+    return np.zeros(np.asarray(d_cdelt1).size, dtype=bool)

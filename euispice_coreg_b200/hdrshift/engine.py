@@ -415,11 +415,26 @@ class LagSearchEngine:
         grid of the small one through the solar-surface change of observer (`coreg_surface_cut`), float64; the
         edge-padded small image and the grid's trig planes for the bilinear per-lag search. `frames`:
         `_ext.CoregSurfaceFrames`. Restated third-party algorithm, parity unpinned (oracle/surface_reproject.py)."""
+        self.set_surface_large(data_large, wcs_large)
+        self.cut_surface(wcs_small, frames)
+        self.d_large_pad = None
+
+    def set_surface_large(self, data_large, wcs_large: TanWcs):
+        """Upload the large image once and edge-pad it once; it stays resident for any number of `cut_surface` calls
+        (frame sequences)."""
         torch = _torch()
         with torch.cuda.device(self.device):
             d_large = self._upload(self._native_float(data_large))
-            self.ref = _ext.surface_cut(wcs_small, wcs_large, _ext.pad_edge(d_large), frames)
+            self.d_large_pad = _ext.pad_edge(d_large)
             del d_large
+        self.wcs_large = wcs_large
+
+    def cut_surface(self, wcs_small: TanWcs, frames):
+        """Per-pair part of the "sunpy" search, after `set_small`: the resident padded large image cut onto the small
+        grid, the grid's trig planes and the edge-padded small image."""
+        torch = _torch()
+        with torch.cuda.device(self.device):
+            self.ref = _ext.surface_cut(wcs_small, self.wcs_large, self.d_large_pad, frames)
             lng, lat = _ext.tan_pix2world(wcs_small, wcs_small.naxis1, wcs_small.naxis2, True, self.device)
             self.planes = _ext.tan_trig_planes(lng, lat, wcs_small.crval1)
             del lng, lat
@@ -632,6 +647,32 @@ class LagSearchEngine:
             self.flagged_lags = k
         return k
 
+    def evaluate_patch_ordered(self, table, lag_ij, planes, return_nvalid=False, pinned=False):
+        """Carrington frame, on this device alone: host offset table [n, 2] -> device corr [n] (and nvalid [n] or
+        None), in the order of `table`. The lags are handed to the kernel in `offset_patch_order` of their grid indices
+        lag_ij = (i1, i2[, group]) and scattered back. Asynchronous; pinned=True stages the uploads in page-locked
+        memory so that the host does not wait for the stream."""
+        torch = _torch()
+        slot, n_slots = offset_patch_order(*lag_ij)
+        padded = np.full((n_slots, table.shape[1]), np.nan, dtype=np.float64)
+        padded[slot] = table
+        with torch.cuda.device(self.device):
+            tab_dev = self._upload(padded, pinned=pinned)
+            idx = self._upload(slot, pinned=pinned)
+            out = torch.empty(n_slots, dtype=torch.float64, device=self.device)
+            nv = torch.empty(n_slots, dtype=torch.int64, device=self.device) if return_nvalid else None
+            self.evaluate(tab_dev, out, nv, planes)
+            return out.index_select(0, idx), (nv.index_select(0, idx) if return_nvalid else None)
+
+    def adopt_reference(self, other):
+        """Search against `other`'s resident reference on the common grid (Carrington frame: one projection shared by
+        the engines of a frame sequence): the same tensor and its statistics column."""
+        torch = _torch()
+        with torch.cuda.device(self.device):
+            self.ref = other.ref
+            self.stats[:, 0].copy_(other.stats[:, 0])
+        self.frame = other.frame
+
     def search(self, table, planes=None, return_nvalid=False, lag_ij=None):
         """Host lag table [n_lags, k] -> numpy corr[n_lags]; shards over ranks when torch.distributed is up.
         lag_ij = (i1, i2[, group]): CRVAL1 / CRVAL2 grid indices of every lag (Carrington frame): each rank's slice is
@@ -645,17 +686,11 @@ class LagSearchEngine:
             local = torch.full((chunk,), float("nan"), dtype=torch.float64, device=self.device)
             nvalid = torch.zeros(chunk, dtype=torch.int64, device=self.device) if return_nvalid else None
             if hi > lo and lag_ij is not None and self.frame == "carrington":
-                slot, n_slots = offset_patch_order(*(np.asarray(v)[lo:hi] for v in lag_ij))
-                padded = np.full((n_slots, table.shape[1]), np.nan, dtype=np.float64)
-                padded[slot] = table[lo:hi]
-                tab_dev = self._upload(padded)
-                out = torch.empty(n_slots, dtype=torch.float64, device=self.device)
-                nv = torch.empty(n_slots, dtype=torch.int64, device=self.device) if return_nvalid else None
-                self.evaluate(tab_dev, out, nv, planes)
-                idx = torch.from_numpy(slot).to(self.device)
-                local[:hi - lo] = out.index_select(0, idx)
+                out, nv = self.evaluate_patch_ordered(table[lo:hi], [np.asarray(v)[lo:hi] for v in lag_ij], planes,
+                                                      return_nvalid=return_nvalid)
+                local[:hi - lo] = out
                 if return_nvalid:
-                    nvalid[:hi - lo] = nv.index_select(0, idx)
+                    nvalid[:hi - lo] = nv
             elif hi > lo:
                 tab_dev = self._upload(table[lo:hi])
                 nv = None if nvalid is None else nvalid[:hi - lo]

@@ -2,10 +2,12 @@
 
 Host file-walking driver (SURVEY.md section 8f rank 1): the list of frames is cut into overlapping sublists; every
 frame of a sublist is co-aligned with the sublist's first frame -- which, from the second sublist on, is the
-CORRECTED file the previous sublist wrote -- and written out with its corrected header. Every co-alignment is one
-`Alignment` search on the device (Carrington grid by default, like the reference). The chain between sublists is
-sequential by construction; `hdrshift/sequence.py::SequenceAlignment` is the batched form for frames that share one
-reference. The reference's "before the reference frame" loop (`:141-174`) can only ever see the single-element
+CORRECTED file the previous sublist wrote -- and written out with its corrected header. The frames of a sublist share
+its reference, so they are searched by one `hdrshift/sequence.py::SequenceAlignment` call (Carrington grid by default,
+like the reference, or helioprojective): the reference is read, uploaded and, in the Carrington frame, projected once
+per sublist instead of once per frame; every cube, and so every file written, is the one of the per-frame `Alignment`.
+Co-alignment of Carrington maps ("initial_carrington") stays one `Alignment` per frame. The chain between sublists is
+sequential by construction: all files of a sublist are written before the next sublist reads its reference. The reference's "before the reference frame" loop (`:141-174`) can only ever see the single-element
 sublist [0] (`idx_list[idx_list[0]::-1]` with `idx_list[0] == 0`) and would raise a NameError on anything longer;
 it is kept as the no-op it is.
 """
@@ -19,6 +21,7 @@ import numpy as np
 
 from .._compat import timeutil
 from ..hdrshift.alignment import Alignment
+from ..hdrshift.sequence import SequenceAlignment
 from ..utils import Util
 
 
@@ -64,7 +67,26 @@ def jitter_correction_imagers(
         path_reference = os.path.join(path_files_output, os.path.basename(list_files_input[index_ref]))
         if ii == 0:
             shutil.copyfile(list_files_input[index_ref], path_reference)
-        for index_to_align in list_[1:]:
+        frames = list_[1:]
+        if alignement_method in ("carrington", "helioprojective") and len(frames):
+            # every frame of the sublist against the one reference: one batched search, reference resident
+            seq = SequenceAlignment(path_reference, [list_files_input[i] for i in frames],
+                                    large_fov_window=window_files_input, small_fov_window=window_files_input,
+                                    small_fov_value_max=small_fov_value_max, small_fov_value_min=small_fov_value_min,
+                                    unit_lag=unit_lag, **parameter_alignment)
+            if alignement_method == "carrington":
+                batch = seq.align_using_carrington(reference_date=dates_files_input[index_ref],
+                                                   method_carrington_reprojection=method_carrington_reprojection,
+                                                   **kwargs_carrington)
+            else:
+                batch = seq.align_using_helioprojective()
+            for index_to_align, results in zip(frames, batch):
+                _plot_correlation(results, path_figures, _hms(dates_files_input[index_to_align]),
+                                  _hms(dates_files_input[index_ref]))
+                _write_corrected(results, list_files_input[index_to_align], window_files_input, path_files_output)
+                all_results.append(results)
+            continue
+        for index_to_align in frames:
             results = _align_hrieuv_with_hrieuv(
                 path_output_figures=path_figures, large_fov_fits_path=path_reference,
                 large_fov_window=window_files_input, small_fov_path=list_files_input[index_to_align],
@@ -74,9 +96,7 @@ def jitter_correction_imagers(
                 reference_date=dates_files_input[index_ref], parallelism=parallelism,
                 alignement_method=alignement_method, small_fov_value_max=small_fov_value_max,
                 small_fov_value_min=small_fov_value_min, unit_lag=unit_lag, **kwargs_carrington)
-            basename_new = os.path.basename(list_files_input[index_to_align])
-            results.write_corrected_fits(window_list_to_apply_shift=[window_files_input],
-                                         path_to_l3_output=os.path.join(path_files_output, basename_new))
+            _write_corrected(results, list_files_input[index_to_align], window_files_input, path_files_output)
             all_results.append(results)
     return all_results
 
@@ -104,10 +124,19 @@ def _align_hrieuv_with_hrieuv(large_fov_fits_path: str, large_fov_window, small_
         results = a.align_using_helioprojective(method="correlation", fov_limits=fov_limits)
     else:
         raise ValueError("alignement_method must be 'carrington', 'initial_carrington' or 'helioprojective'")
+    _plot_correlation(results, path_output_figures, date_to_align, date_ref)
+    return results
+
+
+def _plot_correlation(results, path_output_figures, date_to_align, date_ref):
     if path_output_figures is not None:
         try:
             results.plot_correlation(
                 path_save_figure=os.path.join(path_output_figures, f"correlation_{date_to_align}_{date_ref}.pdf"))
         except ImportError:
             warnings.warn("matplotlib is not installed: no correlation figure written")
-    return results
+
+
+def _write_corrected(results, path_input, window, path_files_output):
+    results.write_corrected_fits(window_list_to_apply_shift=[window],
+                                 path_to_l3_output=os.path.join(path_files_output, os.path.basename(path_input)))
