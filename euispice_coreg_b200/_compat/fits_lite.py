@@ -7,7 +7,9 @@ string/logical/int/float cards, CONTINUE-less headers. Tile-compressed images (`
 `ZCMPTYPE = 'RICE_1'`, the form real Solar Orbiter L2 files come in; `utils/Util.py:144-145`) are read as
 `CompImageHDU`: the header is folded back to an image header on the host, the pixels are decoded ON THE GPU
 (`coreg_rice_decode`, one thread per tile) the first time `.data` is touched, so only the compressed heap crosses
-PCIe. Writing is always uncompressed.
+PCIe. Writing is uncompressed, except for a `CompImageHDU.with_header` copy: it is written as a tile-compressed image
+whose table and heap are the ones read, with the new image header folded back into the table header (no decoding,
+no encoding, no GPU).
 
 If astropy is importable the caller may still hand astropy headers to the package: everything
 downstream only needs the mapping protocol (`in`, `[]`, `.copy()`, `.keys()`).
@@ -306,6 +308,16 @@ class PrimaryHDU(ImageHDU):
 _TFORM_BYTES = {"L": 1, "X": 1, "B": 1, "I": 2, "J": 4, "K": 8, "A": 1, "E": 4, "D": 8, "C": 8, "M": 16, "P": 8, "Q": 16}
 _Z_DROP = ("ZIMAGE", "ZCMPTYPE", "ZQUANTIZ", "ZDITHER0", "ZBLANK", "ZSCALE", "ZZERO", "TFIELDS", "THEAP", "ZMASKCMP",
            "ZSIMPLE", "ZEXTEND", "ZBLOCKED", "ZHECKSUM", "ZDATASUM", "CHECKSUM", "DATASUM")
+_TABLE_CARDS = {"XTENSION", "BITPIX", "NAXIS", "NAXIS1", "NAXIS2", "PCOUNT", "GCOUNT", "ZNAXIS", "ZBITPIX", "ZPCOUNT",
+                "ZGCOUNT", "ZTENSION", *_Z_DROP}
+_TABLE_INDEXED = ("ZNAXIS", "ZTILE", "ZNAME", "ZVAL", "TTYPE", "TFORM", "TUNIT", "TDIM", "TSCAL", "TZERO", "TNULL", "TDISP")
+# cover the header bytes, which a new image header changes; DATASUM / ZDATASUM cover the table and the pixels
+_STALE_CHECKSUMS = ("CHECKSUM", "ZHECKSUM")
+
+
+def _is_table_card(key):
+    """A card of the binary table itself (structure, columns, compression, checksums), not of the image it holds."""
+    return key in _TABLE_CARDS or any(key.startswith(p) and key[len(p):].isdigit() for p in _TABLE_INDEXED)
 
 
 def _tform(tform):
@@ -321,7 +333,10 @@ def _tform(tform):
 
 
 class CompImageHDU:
-    """A tile-compressed image extension. `header` is the image's own header; `data` decodes on first access."""
+    """A tile-compressed image extension. `header` is the image's own header; `data` decodes on first access.
+
+    `writeto` decodes an HDU as read and writes it as a plain IMAGE extension; it writes a `with_header` copy
+    tile-compressed."""
     is_primary = False
 
     def __init__(self, table_header, body):
@@ -329,10 +344,27 @@ class CompImageHDU:
         self._body = body
         self._data = None
         self.header = self._image_header(table_header)
+        self.write_compressed = False
 
     @property
     def name(self):
         return self.header.get("EXTNAME", "")
+
+    @property
+    def table_header(self):
+        """The binary table's header as read: structure, columns, `Z*` compression cards and the image's cards."""
+        return self._thdr
+
+    def with_header(self, header):
+        """The same tiles under the image header `header` (typically a modified `.header.copy()`), to be written by
+        `writeto` as a tile-compressed image: the table and its heap byte for byte as read, the header folded back
+        into the table header (`_table_header`). Neither this HDU nor the copy decodes anything, so no GPU is needed."""
+        if self._body is None:
+            raise OSError("compressed payload already released")
+        out = CompImageHDU(self._thdr, self._body)
+        out.header = header
+        out.write_compressed = True
+        return out
 
     @staticmethod
     def _image_header(th):
@@ -345,18 +377,31 @@ class CompImageHDU:
             h[f"NAXIS{i}"] = int(th[f"ZNAXIS{i}"])
         h["PCOUNT"] = int(th.get("ZPCOUNT", 0))
         h["GCOUNT"] = int(th.get("ZGCOUNT", 1))
-        skip = {"XTENSION", "BITPIX", "NAXIS", "NAXIS1", "NAXIS2", "PCOUNT", "GCOUNT", "ZNAXIS", "ZBITPIX", "ZPCOUNT",
-                "ZGCOUNT", "ZTENSION"}
         for k, (v, c) in th._cards.items():
-            if k in skip or k in _Z_DROP:
-                continue
-            if any(k.startswith(p) and k[len(p):].isdigit() for p in ("ZNAXIS", "ZTILE", "ZNAME", "ZVAL", "TTYPE",
-                                                                          "TFORM", "TUNIT", "TDIM", "TSCAL", "TZERO",
-                                                                          "TNULL", "TDISP")):
-                continue
-            h._cards[k] = (v, c)
+            if not _is_table_card(k):
+                h._cards[k] = (v, c)
         h._commentary = list(th._commentary)
         return h
+
+    @staticmethod
+    def _table_header(th, image_header):
+        """Inverse of `_image_header`: the table header `th` with its image cards replaced by those of `image_header`.
+        The table's own cards (`_is_table_card`) stay as read, in place, except the header checksums CHECKSUM and
+        ZHECKSUM, which are dropped. An image card keeps its place in `th`, takes `image_header`'s value, or goes
+        if `image_header` lacks it; cards new in `image_header` follow the table's cards. Structural image cards
+        (BITPIX, NAXISn, BSCALE, ...) are left out, as `writeto` leaves them out of a plain image's header."""
+        img = OrderedDict((k, vc) for k, vc in image_header._cards.items()
+                          if not (_is_structural(k) or _is_table_card(k)))
+        out = Header()
+        for k, vc in th._cards.items():
+            if _is_table_card(k):
+                if k not in _STALE_CHECKSUMS:
+                    out._cards[k] = vc
+            elif k in img:
+                out._cards[k] = img.pop(k)
+        out._cards.update(img)
+        out._commentary = list(image_header._commentary)
+        return out
 
     @property
     def data(self):
@@ -605,8 +650,20 @@ def _structural_cards(hdu, primary: bool):
 _STRUCTURAL = {"SIMPLE", "XTENSION", "BITPIX", "NAXIS", "EXTEND", "PCOUNT", "GCOUNT", "BSCALE", "BZERO"}
 
 
+def _is_structural(key):
+    """A card `writeto` derives from the data of an image HDU rather than copying it from the header."""
+    return key in _STRUCTURAL or (key.startswith("NAXIS") and key[5:].isdigit())
+
+
+def _header_bytes(cards, commentary):
+    raw = "".join([*cards, *(f"{k:<8}{txt}"[:CARD].ljust(CARD) for k, txt in commentary), "END".ljust(CARD)])
+    raw = raw.encode("ascii", errors="replace")
+    return raw + b" " * ((-len(raw)) % BLOCK)
+
+
 def writeto(path, hdus, overwrite=False):
-    """Write an `HDUList` (or a single HDU) as an uncompressed FITS file."""
+    """Write an `HDUList` (or a single HDU) as a FITS file: image HDUs uncompressed, `CompImageHDU`s as read decoded
+    to plain IMAGE extensions, `CompImageHDU.with_header` copies as tile-compressed images."""
     path = os.fspath(path)
     if os.path.exists(path) and not overwrite:
         raise OSError(f"File {path!r} already exists.")
@@ -615,17 +672,21 @@ def writeto(path, hdus, overwrite=False):
     out = bytearray()
     for idx, hdu in enumerate(hdus):
         primary = idx == 0
+        if isinstance(hdu, CompImageHDU) and hdu.write_compressed:
+            if primary:
+                raise ValueError("a tile-compressed image cannot be the primary HDU")
+            if hdu._body is None:
+                raise OSError("compressed payload already released")
+            th = CompImageHDU._table_header(hdu.table_header, hdu.header)
+            out += _header_bytes([_format_card(k, v, c) for k, (v, c) in th._cards.items()], th._commentary)
+            out += hdu._body + b"\0" * ((-len(hdu._body)) % BLOCK)
+            continue
         cards = [_format_card(k, v, c) for k, v, c in _structural_cards(hdu, primary)]
         for k, (v, c) in hdu.header._cards.items():
-            if k in _STRUCTURAL or (k.startswith("NAXIS") and k[5:].isdigit()):
+            if _is_structural(k):
                 continue
             cards.append(_format_card(k, v, c))
-        for k, txt in hdu.header._commentary:
-            cards.append(f"{k:<8}{txt}"[:CARD].ljust(CARD))
-        cards.append("END".ljust(CARD))
-        raw = "".join(cards).encode("ascii", errors="replace")
-        raw += b" " * ((-len(raw)) % BLOCK)
-        out += raw
+        out += _header_bytes(cards, hdu.header._commentary)
         if hdu.data is not None:
             d = np.ascontiguousarray(hdu.data)
             d = d.astype(d.dtype.newbyteorder(">"))

@@ -25,6 +25,14 @@ def _fits():
         return fits_lite
 
 
+def _is_float32_rice(hdu):
+    """A fits_lite RICE_1 tile-compressed float32 image: its tiles decode to the `<f4` pixels a corrected copy holds."""
+    if not isinstance(hdu, fits_lite.CompImageHDU):
+        return False
+    th = hdu.table_header
+    return str(th.get("ZCMPTYPE", "")).strip().upper() in ("RICE_1", "RICE_ONE") and int(th["ZBITPIX"]) == -32
+
+
 class AlignCommonUtil:
 
     @staticmethod
@@ -138,7 +146,16 @@ class AlignCommonUtil:
     def write_corrected_fits(path_to_l2_input: str, window_list_to_apply_shift, path_to_l3_output: str, corr,
                              lag_crval1=None, lag_crval2=None, lag_crota=None, lag_cdelt1=None, lag_cdelt2=None,
                              shift_arcsec=None):
-        """Copy the input FITS, correcting the headers of the selected windows (`utils/Util.py:106-159`)."""
+        """Copy the input FITS, correcting the headers of the selected windows (`utils/Util.py:106-159`).
+
+        The reference writes a selected window's pixels as `np.array(data, dtype="<f4")`. Without astropy, a selected
+        RICE_1 tile-compressed window with ZBITPIX = -32 decodes to exactly those float32 values, so it is written as
+        a tile-compressed image: the corrected header folded into the table header, the table and the heap byte for
+        byte as read (`fits_lite.CompImageHDU.with_header`). Nothing is decoded, quantised or encoded, and no GPU is
+        needed. astropy would re-quantise the pixels when it re-compresses such a window; that output is not restated
+        here, because neither astropy nor cfitsio is a dependency it could be pinned against. Any other selected
+        compressed window is decoded (on the GPU) and written as a float32 IMAGE extension holding the `<f4` cast.
+        A compressed HDU that is not selected is, as before, decoded and written as a plain image."""
         fits = _fits()
         if shift_arcsec is None:
             max_index = np.unravel_index(np.nanargmax(corr), corr.shape)
@@ -153,15 +170,19 @@ class AlignCommonUtil:
                 if (extname in window_list_to_apply_shift) or (ii in window_list_to_apply_shift) or \
                         ((ii - len(hdul)) in window_list_to_apply_shift):
                     header = hdu.header.copy()
-                    data = hdu.data.copy()
                     AlignCommonUtil.correct_pointing_header(
                         header, lag_crval1=shift_arcsec[0], lag_crval2=shift_arcsec[1], lag_cdelt1=shift_arcsec[2],
                         lag_cdelt2=shift_arcsec[3], lag_crota=shift_arcsec[4])
-                    data = np.array(data, dtype="<f4")
-                    # HDU kind preserved (Primary / Image / CompImage when astropy provides it)
-                    hdu_out = type(hdu)(data=data, header=header)
-                    if hasattr(hdu_out, "verify"):
-                        hdu_out.verify("silentfix")
+                    if _is_float32_rice(hdu):
+                        # never touches `.data`: decoding would release the compressed tiles
+                        hdu_out = hdu.with_header(header)
+                    else:
+                        data = np.array(hdu.data.copy(), dtype="<f4")
+                        # HDU kind preserved (Primary / Image / CompImage when astropy provides it)
+                        cls = fits_lite.ImageHDU if isinstance(hdu, fits_lite.CompImageHDU) else type(hdu)
+                        hdu_out = cls(data=data, header=header)
+                        if hasattr(hdu_out, "verify"):
+                            hdu_out.verify("silentfix")
                     n_corrected += 1
                 else:
                     hdu_out = hdu
