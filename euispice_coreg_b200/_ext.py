@@ -19,12 +19,13 @@ F32, F64, I32 = 0, 1, 2
 FLAG_STRICT = 1
 FLAG_NO_FAST = 4
 FLAG_MIXED = 8      # coreg_hpc_search_host: opt in to the mixed-arithmetic kernel (float32 small payload, guarded)
+FLAG_PURE_SHIFT = 0x100   # every lag is a pure CRVAL shift: the rolling kernel without the adaptive segment
 
 
-def make_flags(strict=False, variant=0, no_fast=False):
+def make_flags(strict=False, no_fast=False, pure_shift=False):
     """flags word of the lag kernels: bit 0 strict scipy op order, bit 2 force the generic kernel,
-    bits 8..11 tuning variant."""
-    return (FLAG_STRICT if strict else 0) | (FLAG_NO_FAST if no_fast else 0) | ((int(variant) & 15) << 8)
+    bit 8 the rolling kernel's flavour for lag grids of pure CRVAL shifts (other kernels ignore it)."""
+    return (FLAG_STRICT if strict else 0) | (FLAG_NO_FAST if no_fast else 0) | (FLAG_PURE_SHIFT if pure_shift else 0)
 
 
 class CoregLibraryError(RuntimeError):

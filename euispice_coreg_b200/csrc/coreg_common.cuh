@@ -30,6 +30,10 @@ inline int fail(int code, const char* fmt, const char* a = "", const char* b = "
 inline int cuda_fail(cudaError_t e, const char* where) {
   return fail(COREG_ECUDA, "%s: %s", where, cudaGetErrorString(e));
 }
+// flags bits 9..11 are reserved: a lag-correlation entry point refuses them before any CUDA call
+inline int check_lag_flags(int flags, const char* entry) {
+  return (flags & 0xE00) ? fail(COREG_EINVAL, "%s: reserved flag bits (9..11) set", entry) : COREG_OK;
+}
 #define CK(call)                                         \
   do {                                                   \
     cudaError_t _e = (call);                             \
@@ -240,15 +244,18 @@ constexpr int kRowsPerPass = kThreads / kTileW;  // 4 grid rows per pass of the 
 constexpr int kWarps = kThreads / 32;
 constexpr int kLagSub = 64;   // lags staged in shared memory at a time
 constexpr int kMom = 8;       // n, Sa, Sb, Saa, Sbb, Sab, pad, pad  (64 B per (tile, lag) partial)
-constexpr int kMinTileH = 16; // smallest tile height of any variant (workspace sizing)
+constexpr int kMinTileH = 16; // tile height of the generic kernel (4 pixels per thread): sizes its partials
 
-constexpr int kRollWRows = 12;  // smallest rows-per-thread of the rolling kernel (tile height 48): sizes the workspace
+// rows per thread the rolling kernel's record rows are laid out for (tiles of 48 grid rows, more record rows than the
+// kernel's 16-row tiles write): sizes the workspace only
+constexpr int kRollWorkspaceRows = 12;
 struct RollWLayout {
   size_t rows, rec, corr, cst, mask, total;   // byte offsets into the workspace
 };
 inline RollWLayout rollw_layout(int gnx, int gny, int64_t n_lags) {
   RollWLayout L;
-  const size_t tiles = (size_t)((gnx + kTileW - 1) / kTileW) * ((gny + 4 * kRollWRows - 1) / (4 * kRollWRows));
+  const size_t tiles = (size_t)((gnx + kTileW - 1) / kTileW) *
+                       ((gny + 4 * kRollWorkspaceRows - 1) / (4 * kRollWorkspaceRows));
   L.rows = tiles * (kThreads / 32);
   L.rec = 0;
   L.corr = L.rec + L.rows * (size_t)n_lags * 3 * sizeof(double);
@@ -422,8 +429,8 @@ inline bool lag_grid(int tile_h, int minb, int gnx, int gny, int64_t n_lags, int
   const int tiles = ((gnx + kTileW - 1) / kTileW) * ((gny + tile_h - 1) / tile_h);
   *tiles_out = tiles;
   // many more blocks than resident slots: border tiles take the per-pixel path and run longer, so a fine
-  // granularity keeps the last wave short (COREG_WAVES overrides the default for tuning)
-  static const int waves = []() { const char* e = getenv("COREG_WAVES"); const int v = e ? atoi(e) : 0; return v > 0 ? v : 128; }();
+  // granularity keeps the last wave short
+  constexpr int waves = 128;
   const int want_blocks = sms * minb * waves;
   int splits = (want_blocks + tiles - 1) / tiles;
   const int max_splits = (int)((n_lags + lag_sub - 1) / lag_sub);

@@ -156,22 +156,20 @@ int launch_finalize_tiles(const double* work, int tiles, int64_t n_lags, double*
   return COREG_OK;
 }
 
-// generic kernel: variant 1 = 8 pixels per thread, 2 CTAs / SM; anything else 4 pixels per thread, 4 CTAs / SM
+// generic kernel: 4 pixels per thread, 4 CTAs / SM. (Measured and dropped: 8 pixels per thread at 2 CTAs / SM,
+// 115.7 vs 101.9 ms on 2048 x 1024 Carrington maps with 3600 lags, profiles/r1_widened_kernels.md.)
 template <class Coord, int ORDER, bool STRICT, typename SmallT, typename RefT, bool ROUND32>
-int launch_lag_variant(int variant, dim3 grid_tiles_of, int gnx, int gny, int64_t n_lags, int sms, cudaStream_t s,
-                       const RefT* ref, const SmallT* small, int snx, int sny, typename Coord::Planes planes,
-                       const typename Coord::Lag* lags, const double* pivots, double* w, int* tiles_out) {
-  (void)grid_tiles_of;
-  const int ppt = (variant == 1) ? 8 : 4, minb = (variant == 1) ? 2 : 4;
+int launch_lag(int gnx, int gny, int64_t n_lags, int sms, cudaStream_t s, const RefT* ref, const SmallT* small, int snx,
+               int sny, typename Coord::Planes planes, const typename Coord::Lag* lags, const double* pivots, double* w,
+               int* tiles_out) {
+  constexpr int PPT = 4, MINB = 4;
+  static_assert(kRowsPerPass * PPT == kMinTileH, "the partials are sized for this tile height");
   dim3 grid;
   int lags_per_block;
-  if (!lag_grid(kRowsPerPass * ppt, minb, gnx, gny, n_lags, sms, &grid, &lags_per_block, tiles_out, kLagSub))
+  if (!lag_grid(kRowsPerPass * PPT, MINB, gnx, gny, n_lags, sms, &grid, &lags_per_block, tiles_out, kLagSub))
     return fail(COREG_EINVAL, "lag grid too large for one launch");
-#define LV(PPT_, MINB_)                                                                                     \
-  lag_corr_kernel<Coord, ORDER, STRICT, SmallT, RefT, ROUND32, PPT_, MINB_><<<grid, kThreads, 0, s>>>(      \
-      ref, small, snx, sny, gnx, gny, planes, lags, (int)n_lags, lags_per_block, pivots, w)
-  if (variant == 1) LV(8, 2); else LV(4, 4);
-#undef LV
+  lag_corr_kernel<Coord, ORDER, STRICT, SmallT, RefT, ROUND32, PPT, MINB><<<grid, kThreads, 0, s>>>(
+      ref, small, snx, sny, gnx, gny, planes, lags, (int)n_lags, lags_per_block, pivots, w);
   return COREG_OK;
 }
 
@@ -187,7 +185,6 @@ int launch_lag_corr(const RefT* ref, const SmallT* small, int snx, int sny, int 
   int sms = coreg_device_sm_count();
   if (sms <= 0) sms = 148;
   const bool strict = (flags & COREG_FLAG_STRICT) != 0;
-  const int variant = (flags >> 8) & 15;
   double* w = static_cast<double*>(work);
   // window kernel for the offset (Carrington) functor: order 2, FMA arithmetic, image of at least 3x3
   const bool fast_ok = std::is_same<Coord, OffsetCoord>::value && (order == 2) && !strict && snx >= 3 && sny >= 3 &&
@@ -206,9 +203,9 @@ int launch_lag_corr(const RefT* ref, const SmallT* small, int snx, int sny, int 
     CK(cudaEventRecord(g_prof[g_prof_n].a, s));
   }
   int tiles = 0, rc = COREG_OK;
-#define LAUNCH(ORD, STR)                                                                                          \
-  rc = launch_lag_variant<Coord, ORD, STR, SmallT, RefT, ROUND32>(variant, dim3(), gnx, gny, n_lags, sms, s, ref, \
-                                                                   small, snx, sny, planes, lags, pivots, w, &tiles)
+#define LAUNCH(ORD, STR)                                                                                         \
+  rc = launch_lag<Coord, ORD, STR, SmallT, RefT, ROUND32>(gnx, gny, n_lags, sms, s, ref, small, snx, sny, planes, \
+                                                          lags, pivots, w, &tiles)
   switch (order) {
     case 0: LAUNCH(0, true); break;
     case 1: LAUNCH(1, true); break;
@@ -250,6 +247,7 @@ int coreg_hpc_lag_corr(const float* ref, const void* small, int small_dtype, int
                        void* stream) {
   if (!ref || !small || !planes || !lags || !pivots || !work || !corr)
     return fail(COREG_EINVAL, "coreg_hpc_lag_corr: null pointer");
+  if (int rc = check_lag_flags(flags, "coreg_hpc_lag_corr")) return rc;
   TanCoord::Planes pl{planes, (int64_t)gnx * gny};
   cudaStream_t s = (cudaStream_t)stream;
   if (small_dtype == COREG_F64)
@@ -268,6 +266,7 @@ int coreg_hpc_lag_corr_edge(const double* ref, const double* small_pad, int snx,
                             void* work, size_t work_bytes, double* corr, int64_t* nvalid, int flags, void* stream) {
   if (!ref || !small_pad || !planes || !lags || !pivots || !work || !corr)
     return fail(COREG_EINVAL, "coreg_hpc_lag_corr_edge: null pointer");
+  if (int rc = check_lag_flags(flags, "coreg_hpc_lag_corr_edge")) return rc;
   if (n_lags <= 0) return COREG_OK;
   if (n_lags > (int64_t)1 << 30) return fail(COREG_EINVAL, "too many lags in one call (max 2^30)");
   if (gnx <= 0 || gny <= 0 || snx <= 0 || sny <= 0) return fail(COREG_EINVAL, "empty image");
@@ -286,9 +285,8 @@ int coreg_hpc_lag_corr_edge(const double* ref, const double* small_pad, int snx,
     CK(cudaEventRecord(g_prof[g_prof_n].a, s));
   }
   // bilinear, scipy's operation order (what reproject calls), float64 reference, no float32 store
-  int rc = launch_lag_variant<TanEdgeCoord, 1, true, double, double, false>((flags >> 8) & 15, dim3(), gnx, gny, n_lags,
-                                                                            sms, s, ref, small_pad, pnx, pny, pl, lags,
-                                                                            pivots, static_cast<double*>(work), &tiles);
+  int rc = launch_lag<TanEdgeCoord, 1, true, double, double, false>(gnx, gny, n_lags, sms, s, ref, small_pad, pnx, pny,
+                                                                    pl, lags, pivots, static_cast<double*>(work), &tiles);
   if (rc) return rc;
   CK_LAUNCH("lag_corr_kernel<TanEdgeCoord>");
   if (prof) {
@@ -304,6 +302,7 @@ int coreg_offset_lag_corr(const double* ref, const void* small, int small_dtype,
                           int flags, void* stream) {
   if (!ref || !small || !tx || !ty || !lags || !pivots || !work || !corr)
     return fail(COREG_EINVAL, "coreg_offset_lag_corr: null pointer");
+  if (int rc = check_lag_flags(flags, "coreg_offset_lag_corr")) return rc;
   OffsetCoord::Planes pl{tx, ty};
   cudaStream_t s = (cudaStream_t)stream;
   if (small_dtype == COREG_F64)
@@ -322,6 +321,7 @@ int coreg_car_lag_corr(const float* ref, const void* small, int small_dtype, int
                        void* work, size_t work_bytes, double* corr, int64_t* nvalid, int flags, void* stream) {
   if (!ref || !small || !planes || !lags || !pivots || !work || !corr)
     return fail(COREG_EINVAL, "coreg_car_lag_corr: null pointer");
+  if (int rc = check_lag_flags(flags, "coreg_car_lag_corr")) return rc;
   CarCoord::Planes pl{planes, (int64_t)gnx * gny};
   cudaStream_t s = (cudaStream_t)stream;
   if (small_dtype == COREG_F64)

@@ -30,13 +30,11 @@
 
 #include "coreg_common.cuh"
 
-#ifndef COREG_OFF_UNROLL
-#define COREG_OFF_UNROLL 2     // pixels of the walk in flight per lane (tuning: tools/carr_lab.py with COREG_LIB_PATH)
-#endif
-
 namespace coreg {
 
 constexpr int kOffThreads = 256;          // = lags per chunk (one lag per thread)
+constexpr int kOffMinBlocks = 3;          // resident blocks per SM (__launch_bounds__)
+constexpr int kOffUnroll = 2;             // pixels of the walk in flight per lane (timed with tools/carr_lab.py)
 constexpr int kOffWarps = kOffThreads / 32;
 constexpr int kOffTileW = 32, kOffTileH = 8, kOffTilePx = kOffTileW * kOffTileH;   // one pixel per thread
 constexpr int kOffTilesPerBlock = 8;      // stacked vertically: super-tile = 32 x 64 grid pixels
@@ -249,8 +247,7 @@ __device__ __forceinline__ void offset_walk_window(unsigned win, int lo_x, int l
                                                    double& sbb, double& sab, int& n_miss, double& sa_miss,
                                                    double& saa_miss, int& n_out, int& n_exact) {
   constexpr int ROW = OffBox<T>::W * (int)sizeof(T), E = (int)sizeof(T);
-  constexpr int kUnroll = COREG_OFF_UNROLL;
-#pragma unroll kUnroll
+#pragma unroll kOffUnroll
   for (int k = 0; k < n_live; ++k, px += (unsigned)sizeof(OffPx)) {
     double ptx, pty, ac;
     lds_px(px, ptx, pty, ac);
@@ -359,11 +356,8 @@ __device__ __forceinline__ bool dirty_value(double v) {
   return (((unsigned)__double2hiint(v) & 0x7FF00000u) == 0x7FF00000u) || (v == -32762.0);
 }
 
-#ifndef COREG_OFF_MINB
-#define COREG_OFF_MINB 3
-#endif
 template <typename T>
-__global__ void __launch_bounds__(kOffThreads, COREG_OFF_MINB)
+__global__ void __launch_bounds__(kOffThreads, kOffMinBlocks)
 offset_window_kernel(const __grid_constant__ CUtensorMap tmap, int use_tma, const double* __restrict__ ref,
                      const T* __restrict__ small, int snx, int sny, int gnx, int gny, const double* __restrict__ tx,
                      const double* __restrict__ ty, const CoregLagOffset* __restrict__ lags, int n_lags,

@@ -449,10 +449,7 @@ __device__ __forceinline__ bool roll_segment_adaptive(const double* __restrict__
   return (bmax < 0x7F800000u) && (((unsigned)__double2hiint(sbb) & 0x7FF00000u) != 0x7FF00000u);
 }
 
-#ifndef COREG_ADAPT_MIN
-#define COREG_ADAPT_MIN 1
-#endif
-constexpr int kAdaptMin = COREG_ADAPT_MIN;   // irregular lanes from which the whole warp takes the adaptive segment (measured 1 / 3 / 6: 15.0 / 15.7 / 16.6 us per lag)
+constexpr int kAdaptMin = 1;   // irregular lanes from which the whole warp takes the adaptive segment (measured 1 / 3 / 6: 15.0 / 15.7 / 16.6 us per lag)
 
 // One pixel by the per-pixel rules: own floors, 9 taps when they are all inside the image, otherwise the exact
 // out-of-line sampler. (sx, sy) are the coordinates + 0.5. Returns false when the sample is missing.
@@ -731,10 +728,7 @@ __device__ __forceinline__ void roll_pixels_warp(unsigned need, const HomLag& C,
   }
 }
 
-#ifndef COREG_ROLL_CHUNK
-#define COREG_ROLL_CHUNK 8
-#endif
-constexpr int kRollChunk = COREG_ROLL_CHUNK;  // lags whose per-lane sums wait in a warp's shared-memory slice for one fold
+constexpr int kRollChunk = 8;  // lags whose per-lane sums wait in a warp's shared-memory slice for one fold
 
 // ---------------------------------------------------------------------------------------------------------
 // The rolling kernel proper. Warps are independent: no block barrier inside the lag walk. Every warp keeps its own
@@ -979,29 +973,24 @@ lag_corr_finalize_w_kernel(const double* __restrict__ wrec, const double* __rest
   }
 }
 
-// rolling kernel + its finalize. Tuning variants (flags bits 8..11):
-//   0  16 rows per thread, with the adaptive segment for rotated / rescaled lags (the default)
-//   1  16 rows per thread, without it: for lag grids of pure CRVAL shifts, where no segment drifts. The adaptive code is
-//      never executed there, but its presence in the kernel costs the regular path 1 % (all-FP64) to 3 % (mixed) through
-//      register allocation and code placement -- so the caller that knows its WHOLE lag grid holds shifts only asks for
-//      this flavour (the choice must not depend on how the grid is sharded: both flavours are correct for any lag, but
-//      they round an irregular segment differently)
-//   2  14 rows per thread (all-FP64 only), 3  12 rows per thread with the adaptive segment
-// The workspace layout is sized for 12 rows (fewer rows per thread would need more record rows). small32 != nullptr
-// selects the mixed-arithmetic kernel (FP64 coordinates, FP32 spline on the float32 copy of the small image).
-// (Until the adaptive segment existed, 12 rows were the better shape for rotated / rescaled lags -- fewer irregular
-// segments; with it 16 rows win there too: 14.0 vs 14.4 us per lag on the 5-D grid. Measured and dropped: 3 CTAs per SM
-// at 80 registers -- spills; 24 and 32 rows per thread -- spills and partial tiles; a precomputed row-coefficient
-// plane: tools/mixed_lab.py, profiles/r1_mixed_kernel.md.)
+// rolling kernel + its finalize: 16 rows per thread, 2 CTAs / SM. `adapt` selects the flavour with the adaptive segment
+// for rotated / rescaled lags; without it (COREG_FLAG_PURE_SHIFT) the kernel serves lag grids of pure CRVAL shifts,
+// where no segment drifts. The adaptive code is never executed there, but its presence in the kernel costs the regular
+// path 1 % (all-FP64) to 3 % (mixed) through register allocation and code placement -- so the caller that knows its
+// WHOLE lag grid holds shifts only asks for this flavour (the choice must not depend on how the grid is sharded: both
+// flavours are correct for any lag, but they round an irregular segment differently). small32 != nullptr selects the
+// mixed-arithmetic kernel (FP64 coordinates, FP32 spline on the float32 copy of the small image).
+// (Measured and dropped: 12 and 14 rows per thread -- 40.1 and 39.4 against 37.8 ms on config 1,
+// profiles/r2_k1_tuning.md; with the adaptive segment 16 rows win for rotated / rescaled lags too, 14.0 vs 14.4 us per
+// lag on the 5-D grid against 12 rows; 3 CTAs per SM at 80 registers -- spills; 24 and 32 rows per thread -- spills and
+// partial tiles; a precomputed row-coefficient plane: tools/mixed_lab.py, profiles/r1_mixed_kernel.md.)
 template <typename RefT, bool ROUND32>
-int launch_lag_rollw(int variant, int gnx, int gny, int64_t n_lags, int sms, cudaStream_t s, const RefT* ref,
+int launch_lag_rollw(bool adapt, int gnx, int gny, int64_t n_lags, int sms, cudaStream_t s, const RefT* ref,
                      const double* small, const float* small32, int snx, int sny,
                      const HomLag* ft, const double* pivots, void* work, double* corr, int64_t* nvalid, bool prof,
                      int* flagged) {
+  constexpr int P = 16, MINB = 2;
   const bool mixed = small32 != nullptr;
-  const int minb = 2;
-  if (mixed && variant == 2) variant = 0;
-  const int rows_per_thread = (variant == 3) ? kRollWRows : ((variant == 2) ? 14 : 16);
   const RollWLayout L = rollw_layout(gnx, gny, n_lags);
   char* base = static_cast<char*>(work);
   double* wrec = reinterpret_cast<double*>(base + L.rec);
@@ -1010,30 +999,23 @@ int launch_lag_rollw(int variant, int gnx, int gny, int64_t n_lags, int sms, cud
   unsigned* wmask = reinterpret_cast<unsigned*>(base + L.mask);
   dim3 grid;
   int lpb, tiles;
-  if (!lag_grid(kRowsPerPass * rows_per_thread, minb, gnx, gny, n_lags, sms, &grid, &lpb, &tiles, kRollChunk, true))
+  if (!lag_grid(kRowsPerPass * P, MINB, gnx, gny, n_lags, sms, &grid, &lpb, &tiles, kRollChunk, true))
     return fail(COREG_EINVAL, "lag grid too large for one launch");
   CK(cudaMemsetAsync(wmask, 0, (size_t)tiles * (size_t)n_lags * sizeof(unsigned), s));
   if (prof) CK(cudaEventRecord(g_prof[g_prof_n].a, s));
-#define RW(P_, MIXED_, ADAPT_)                                                                                       \
-  {                                                                                                                  \
-    auto kern = lag_corr_roll_kernel<RefT, ROUND32, P_, 2, MIXED_, ADAPT_>;                                          \
-    cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RollWShared));               \
-    kern<<<grid, kThreads, sizeof(RollWShared), s>>>(ref, small, small32, snx, sny, gnx, gny, ft, (int)n_lags, lpb,  \
-                                                     pivots, wrec, wcorr, wconst, wmask);                            \
-  }
-  if (mixed) {
-    if (variant == 3) RW(kRollWRows, true, true) else if (variant == 1) RW(16, true, false) else RW(16, true, true)
-  } else {
-    if (variant == 3) RW(kRollWRows, false, true) else if (variant == 2) RW(14, false, false)
-    else if (variant == 1) RW(16, false, false) else RW(16, false, true)
-  }
-#undef RW
+  auto kern = mixed ? (adapt ? lag_corr_roll_kernel<RefT, ROUND32, P, MINB, true, true>
+                             : lag_corr_roll_kernel<RefT, ROUND32, P, MINB, true, false>)
+                    : (adapt ? lag_corr_roll_kernel<RefT, ROUND32, P, MINB, false, true>
+                             : lag_corr_roll_kernel<RefT, ROUND32, P, MINB, false, false>);
+  cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(RollWShared));
+  kern<<<grid, kThreads, sizeof(RollWShared), s>>>(ref, small, small32, snx, sny, gnx, gny, ft, (int)n_lags, lpb, pivots,
+                                                   wrec, wcorr, wconst, wmask);
   CK_LAUNCH("lag_corr_roll_kernel");
   if (prof) {
     CK(cudaEventRecord(g_prof[g_prof_n].b, s));
     ++g_prof_n;
   }
-  // record rows actually written: 8 warps per tile of this variant (<= L.rows)
+  // record rows actually written: 8 warps per 16-row tile (<= L.rows)
   // mixed arithmetic: `pivots` is the head of the [4][2] statistics block (coreg_image_stats / coreg_center_f32)
   lag_corr_finalize_w_kernel<<<(unsigned)((n_lags + kRollChunk - 1) / kRollChunk), 256, 0, s>>>(
       wrec, wcorr, wconst, wmask, tiles * kWarps, (int)n_lags, corr, nvalid, (mixed && flagged) ? pivots : nullptr, flagged);
@@ -1059,8 +1041,8 @@ int hpc_lag_corr_wcs_impl(const float* ref, const double* small, const float* sm
     CK(cudaEventCreate(&g_prof[g_prof_n].a));
     CK(cudaEventCreate(&g_prof[g_prof_n].b));
   }
-  return launch_lag_rollw<float, true>((flags >> 8) & 15, gnx, gny, n_lags, sms, s, ref, small, small32, snx, sny, ft,
-                                       pivots, work, corr, nvalid, prof, flagged);
+  return launch_lag_rollw<float, true>(!(flags & COREG_FLAG_PURE_SHIFT), gnx, gny, n_lags, sms, s, ref, small, small32,
+                                       snx, sny, ft, pivots, work, corr, nvalid, prof, flagged);
 }
 }  // namespace coreg
 
@@ -1074,6 +1056,7 @@ int coreg_hpc_lag_corr_wcs(const float* ref, const double* small, int snx, int s
                            int flags, void* stream) {
   if (!ref || !small || !grid_wcs || !lag_wcs || !pivots || !work || !corr)
     return fail(COREG_EINVAL, "coreg_hpc_lag_corr_wcs: null pointer");
+  if (int rc = check_lag_flags(flags, "coreg_hpc_lag_corr_wcs")) return rc;
   if (n_lags <= 0) return COREG_OK;
   if (order != 2 || (flags & COREG_FLAG_STRICT))
     return fail(COREG_EINVAL, "coreg_hpc_lag_corr_wcs: only order 2 with FMA arithmetic; use coreg_hpc_lag_corr");
@@ -1091,6 +1074,7 @@ int coreg_hpc_lag_corr_wcs_mixed(const float* ref, const double* small, const fl
                                  double* corr, int64_t* nvalid, int* flagged, int flags, void* stream) {
   if (!ref || !small || !small32c || !grid_wcs || !lag_wcs || !stats || !work || !corr || !flagged)
     return fail(COREG_EINVAL, "coreg_hpc_lag_corr_wcs_mixed: null pointer");
+  if (int rc = check_lag_flags(flags, "coreg_hpc_lag_corr_wcs_mixed")) return rc;
   if (n_lags <= 0) return COREG_OK;
   if (order != 2 || (flags & COREG_FLAG_STRICT))
     return fail(COREG_EINVAL, "coreg_hpc_lag_corr_wcs_mixed: only order 2 with FMA arithmetic; use coreg_hpc_lag_corr");

@@ -223,8 +223,12 @@ class LagSearchEngine:
         projection, FP32 spline on the pivot-centred float32 payload of the small image; applies to the homography
         kernel when every small-image pixel is a float32 value; lags whose error model exceeds 1e-7 in r are
         re-evaluated in FP64, see `resolve_flags`). None: the COREG_ARITHMETIC environment variable, else
-        `default_arithmetic`."""
+        `default_arithmetic`.
+        variant: flavour of the helioprojective rolling kernel. 0 (default): chosen from the lag grid (`hpc_lag_table`
+        sets `pure_shift_hint`); 1: always the flavour for pure CRVAL shifts (`_ext.FLAG_PURE_SHIFT`)."""
         torch = _torch()
+        if variant not in (0, 1):
+            raise ValueError("variant must be 0 (kernel flavour chosen from the lag grid) or 1 (pure-shift flavour)")
         arithmetic = arithmetic or os.environ.get("COREG_ARITHMETIC") or self.default_arithmetic
         if arithmetic not in ("fp64", "mixed"):
             raise ValueError('arithmetic must be "fp64" or "mixed"')
@@ -239,8 +243,8 @@ class LagSearchEngine:
         self.device = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
         self.order = int(order)
         self.strict = bool(strict)
-        self.variant, self.no_fast = int(variant), bool(no_fast)
-        self.flags = _ext.make_flags(strict, variant, no_fast=no_fast)
+        self.no_fast = bool(no_fast)
+        self.flags = _ext.make_flags(strict, no_fast=no_fast, pure_shift=variant == 1)
         self.small_storage = small_storage
         # statistics block [4, 2]: rows = mean (the pivot), count, max |v|, RMS about the pivot; columns = ref, small
         self.stats = torch.zeros((_ext.STATS_ROWS, 2), dtype=torch.float64, device=self.device)
@@ -471,10 +475,6 @@ class LagSearchEngine:
             self.grid_wcs = wcs_small
             _ext.image_stats(self.ref, self.stats, 0)
         self.frame = "car"
-        # launch shape of the generic kernel: the default 4 pixels x 4 CTAs / SM (64 registers, the atan2 temporaries
-        # spill to L1-resident local memory) measured faster than 8 x 2 with 128 registers: 101.9 vs 115.7 ms on
-        # 2048 x 1024 maps, 3600 lags (profiles/r1_widened_kernels.md)
-        self.flags = _ext.make_flags(self.strict, int(os.environ.get("COREG_CAR_VARIANT", "0")), no_fast=self.no_fast)
 
     def _hpc_planes(self):
         """Lag-independent trig planes of the generic helioprojective kernel (101 MB at 2048^2), built lazily:
@@ -600,10 +600,10 @@ class LagSearchEngine:
                 nv = None if nvalid_dev is None else nvalid_dev[lo:hi]
                 if self.frame == "hpc" and table_dev.shape[1] == _ext.TAN_WCS_DOUBLES:
                     flags = self.flags
-                    if self.variant == 0 and self.pure_shift_hint:
+                    if self.pure_shift_hint:
                         # a grid of pure CRVAL shifts: the kernel flavour without the adaptive segment (1 - 3 % faster
                         # on the regular path, csrc/coreg_lag_roll.cu); decided on the WHOLE lag grid, never on a shard
-                        flags = _ext.make_flags(self.strict, 1, no_fast=self.no_fast)
+                        flags |= _ext.FLAG_PURE_SHIFT
                     _ext.hpc_lag_corr_wcs(self.ref, self.small, self.grid_wcs, table_dev[lo:hi], self.order,
                                           self.stats if mixed else self.pivots, work, out_dev[lo:hi], nv, flags,
                                           small32c=self.small32 if mixed else None,

@@ -36,7 +36,7 @@ extern "C" {
 /* flags of the lag-correlation kernels.
  * Default arithmetic: FP64 with fused multiply-add in the spline weights / tap sums (|dr| ~ 1e-15 vs strict).
  * COREG_FLAG_STRICT: scipy's exact operation order (separate multiply / add), bit-faithful per sample.
- * bits 8..11: tuning variant of the fused kernel (0 = default tile / occupancy; see DESIGN.md). */
+ * Bits 9..11 are reserved: every lag-correlation entry point returns COREG_EINVAL when one is set. */
 #define COREG_FLAG_STRICT 1
 /* COREG_FLAG_NO_FAST (value 4; 2 is reserved): force the generic kernel (testing / comparison). */
 #define COREG_FLAG_NO_FAST 4
@@ -44,7 +44,11 @@ extern "C" {
  * the small image is COREG_F32 and the fast form applies; the entry checks the kernel's per-lag guard and repeats the
  * search in FP64 when any lag trips it. Default (flag clear): all FP64, the reference's arithmetic. */
 #define COREG_FLAG_MIXED 8
-#define COREG_FLAG_VARIANT(v) (((v) & 15) << 8)
+/* COREG_FLAG_PURE_SHIFT: every lag is a pure CRVAL shift; selects the rolling kernel (coreg_hpc_lag_corr_wcs,
+ * coreg_hpc_lag_corr_wcs_mixed) without the adaptive segment; other kernels ignore it. Set it from the WHOLE lag grid:
+ * both flavours are correct for any lag but round an irregular column segment differently, so every part of a sharded
+ * grid must use the same one. */
+#define COREG_FLAG_PURE_SHIFT 0x100
 
 /* Constants of a 2-axis gnomonic (TAN) WCS. Replaces `astropy.wcs.WCS(hdr)`:
  * hdrshift/alignment.py:1041, utils/Util.py:284, synras/map_builder.py:119. */
@@ -274,10 +278,9 @@ int coreg_hpc_lag_corr_wcs(const float* ref_dev, const double* small_dev, int sn
  *                 as float32 (alignment.py:1024); this kernel reproduces that float32 store on the uncentred value,
  *                 so its samples equal the reference's except within a few float32 ulps OF THE DEVIATION FROM THE
  *                 PIVOT of a rounding boundary: |dr| <= 1e-7 by the model, ~1e-10 observed, independent of the image's
- *                 mean level. Variants (COREG_FLAG_VARIANT): 0 = 16 rows per thread with the adaptive segment for
- *                 rotated / rescaled lags (default), 1 = 16 rows without it (lag grids of pure CRVAL shifts: the same
- *                 flavour must then be used for every part of the grid; x is taken as a line in the row index where
- *                 its quadratic term stays below 1e-11 pixel), 3 = 12 rows with it. */
+ *                 mean level. Without COREG_FLAG_PURE_SHIFT the kernel carries the adaptive segment for rotated /
+ *                 rescaled lags; with it the adaptive segment is left out and x is taken as a line in the row index
+ *                 where its quadratic term stays below 1e-11 pixel. */
 int coreg_hpc_lag_corr_wcs_mixed(const float* ref_dev, const double* small_dev, const float* small32c_dev, int snx,
                                  int sny, int gnx, int gny, const CoregTanWcs* grid_wcs_host,
                                  const CoregTanWcs* lag_wcs_dev, int64_t n_lags, int order, const double* stats_dev,

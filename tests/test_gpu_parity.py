@@ -359,7 +359,7 @@ def test_host_buffer_entry_point_matches_device_path(torch_cuda, toy_pair):
     d = engine.flat_lag_grid(LAGS["lag_crval1"], LAGS["lag_crval2"], [0.0], [0.0], [0.0])
     w_small = TanWcs.from_header(a.hdr_small)
     table, _ = engine.tan_wcs_table(a.hdr_small, a, *d)
-    flags = _ext.make_flags(variant=1)    # 16 rows per thread: what the engine launches for a pure CRVAL lag grid
+    flags = _ext.FLAG_PURE_SHIFT    # what the engine launches for a pure CRVAL lag grid
     corr, nvalid = _ext.hpc_search_host(dl.astype(np.float64), TanWcs.from_header(hl), ds.astype(np.float64), w_small,
                                         table, flags=flags)
     assert np.array_equal(corr.reshape(gpu.shape), gpu)
@@ -372,11 +372,11 @@ def test_host_buffer_entry_point_matches_device_path(torch_cuda, toy_pair):
     corr_g, nv_g = _ext.hpc_search_host(dl, TanWcs.from_header(hl), ds, w_small, table,
                                         flags=_ext.make_flags(no_fast=True))
     assert np.nanmax(np.abs(corr_g - corr)) < 1e-11 and np.array_equal(nv_g, nvalid)
-    # mixed arithmetic through the same entry (COREG_FLAG_MIXED, float32 payload; 16 rows per thread is what the
+    # mixed arithmetic through the same entry (COREG_FLAG_MIXED, float32 payload; the pure-shift flavour is what the
     # engine launches for pure CRVAL lags) == the torch-plumbed default path, bit for bit
     gpu_m, a_m = _gpu_cube(toy_pair, arithmetic="mixed", **LAGS)
     corr_m, nv_m = _ext.hpc_search_host(dl, TanWcs.from_header(hl), ds, w_small, table,
-                                        flags=_ext.make_flags(variant=1) | _ext.FLAG_MIXED)
+                                        flags=_ext.FLAG_PURE_SHIFT | _ext.FLAG_MIXED)
     assert np.array_equal(corr_m.reshape(gpu_m.shape), gpu_m) and np.array_equal(nv_m, nvalid)
     assert not np.array_equal(corr_m, corr) and np.nanmax(np.abs(corr_m - corr)) < OBSERVED["mixed"]
     # a float64 payload has no float32 twin on this entry: the flag is ignored, FP64 kernel
@@ -397,7 +397,7 @@ def test_multi_device_host_entry_point_gives_the_same_cube(torch_cuda, toy_pair)
     d = engine.flat_lag_grid(LAGS["lag_crval1"], LAGS["lag_crval2"], [0.0], [0.0], [0.0])
     w_small = TanWcs.from_header(a.hdr_small)
     table, _ = engine.tan_wcs_table(a.hdr_small, a, *d)
-    flags = _ext.make_flags(variant=1)
+    flags = _ext.FLAG_PURE_SHIFT
     one, nv_one = _ext.hpc_search_host(dl, TanWcs.from_header(hl), ds, w_small, table, flags=flags)
     n_dev = torch_cuda.cuda.device_count()
     for devices in ([0, 0, 0], list(range(n_dev)), [0] * 30):      # 30 devices for 25 lags: empty slices
@@ -620,7 +620,7 @@ def test_adaptive_segment_rotated_rescaled_lags_with_holes(torch_cuda, tmp_path)
     lane takes the rolling kernel's ADAPTIVE segment (every pixel its own floors, csrc/coreg_lag_roll.cu). A grid large
     enough to have interior warps (448 x 448: the toy pairs are all rim), NaN holes in the small image (an adaptive
     segment that meets a non-finite sample is redone pixel by pixel), against the oracle; and against the kernel flavour
-    WITHOUT the adaptive code (variant 1), which evaluates the same lags by the per-pixel rules."""
+    WITHOUT the adaptive code (`_ext.FLAG_PURE_SHIFT`), which evaluates the same lags by the per-pixel rules."""
     import torch
     from euispice_coreg_b200 import _ext
     from euispice_coreg_b200._compat import fits_lite
@@ -647,7 +647,7 @@ def test_adaptive_segment_rotated_rescaled_lags_with_holes(torch_cuda, tmp_path)
     table, _ = a.engine.hpc_lag_table(a.hdr_small, a, *d, "intended")
     c0, n0 = a.engine.search(table, return_nvalid=True)
     assert np.array_equal(c0, gpu.ravel())
-    a.engine.variant, a.engine.flags = 1, _ext.make_flags(variant=1)
+    a.engine.flags |= _ext.FLAG_PURE_SHIFT
     c1, n1 = a.engine.search(table, return_nvalid=True)
     # (the float32 store of every sample hides the different FP64 operation order of the two paths: the cubes usually
     # agree to the last bit)

@@ -357,6 +357,24 @@ def test_c_abi_argument_validation_needs_no_device():
     assert rc == EINVAL and "null" in msg()
     rc = lib.coreg_hpc_cut(ctypes.byref(good), 8, 8, ctypes.byref(good), fake, 5, 8, 8, 0, 0, 2, fake, null)
     assert rc == EINVAL and "dtype" in msg()
+    # flags bits 9..11 are reserved: every lag-correlation entry refuses them
+    big, g = 1 << 30, ctypes.byref(good)
+    entries = {
+        "coreg_hpc_lag_corr": lambda f: (fake, fake, _ext.F64, 8, 8, 8, 8, fake, fake, 4, 2, fake, fake, big, fake,
+                                         null, f, null),
+        "coreg_hpc_lag_corr_edge": lambda f: (fake, fake, 8, 8, 8, 8, fake, fake, 4, fake, fake, big, fake, null, f, null),
+        "coreg_offset_lag_corr": lambda f: (fake, fake, _ext.F64, 8, 8, 8, 8, fake, fake, fake, 4, 2, fake, fake, big,
+                                            fake, null, f, null),
+        "coreg_car_lag_corr": lambda f: (fake, fake, _ext.F64, 8, 8, 8, 8, fake, fake, 4, 2, fake, fake, big, fake,
+                                         null, f, null),
+        "coreg_hpc_lag_corr_wcs": lambda f: (fake, fake, 8, 8, 8, 8, g, fake, 4, 2, fake, fake, big, fake, null, f, null),
+        "coreg_hpc_lag_corr_wcs_mixed": lambda f: (fake, fake, fake, 8, 8, 8, 8, g, fake, 4, 2, fake, fake, big, fake,
+                                                   null, fake, f, null),
+    }
+    for name, args in entries.items():
+        for bit in (9, 10, 11):
+            rc = getattr(lib, name)(*args((1 << bit) | _ext.FLAG_PURE_SHIFT))
+            assert rc == EINVAL and msg() == name + ": reserved flag bits (9..11) set", (name, bit, msg())
 
 
 # ----------------------------------------------------------------------------------------------- multi-rank

@@ -1,5 +1,5 @@
 """Where the time of BASELINE configs[3] (1 024 000-lag 5-D grid) goes: host table, upload, device time per lag for
-rotated / rescaled lags at 12 and 16 rows per thread (GPU box).    python tools/grid5d_lab.py [--lags 31744]"""
+rotated / rescaled lags and for pure CRVAL lags of the same count (GPU box).    python tools/grid5d_lab.py [--lags 31744]"""
 import argparse
 import json
 import os
@@ -41,32 +41,28 @@ def main():
     n = min(args.lags, table.shape[0])
     # a representative block: lags spread over the whole grid
     sel = np.linspace(0, table.shape[0] - 1, n).astype(np.int64)
-    for variant in (0, 3):
-        eng.variant = variant
-        eng.flags = _ext.make_flags(False, variant)
-        torch.cuda.synchronize()
-        t3 = time.perf_counter()
-        tab = eng._upload(table[sel])
-        torch.cuda.synchronize()
-        t4 = time.perf_counter()
-        out = torch.empty(n, dtype=torch.float64, device=eng.device)
-        eng.evaluate(tab, out)
-        torch.cuda.synchronize()
-        _ext.profile_begin()
-        t5 = time.perf_counter()
-        eng.evaluate(tab, out)
-        torch.cuda.synchronize()
-        t6 = time.perf_counter()
-        ms, k = _ext.profile_end()
-        print(json.dumps({"variant": variant, "rows_per_thread": 12 if variant == 3 else 16, "lags": n,
-                          "upload_s": t4 - t3, "evaluate_wall_s": t6 - t5, "lag_kernel_ms": ms, "launches": k,
-                          "us_per_lag_kernel": 1e3 * ms / n, "us_per_lag_wall": 1e6 * (t6 - t5) / n}), flush=True)
+    torch.cuda.synchronize()
+    t3 = time.perf_counter()
+    tab = eng._upload(table[sel])
+    torch.cuda.synchronize()
+    t4 = time.perf_counter()
+    out = torch.empty(n, dtype=torch.float64, device=eng.device)
+    eng.evaluate(tab, out)
+    torch.cuda.synchronize()
+    _ext.profile_begin()
+    t5 = time.perf_counter()
+    eng.evaluate(tab, out)
+    torch.cuda.synchronize()
+    t6 = time.perf_counter()
+    ms, k = _ext.profile_end()
+    print(json.dumps({"lags": n, "upload_s": t4 - t3, "evaluate_wall_s": t6 - t5, "lag_kernel_ms": ms, "launches": k,
+                      "us_per_lag_kernel": 1e3 * ms / n, "us_per_lag_wall": 1e6 * (t6 - t5) / n}), flush=True)
     # pure CRVAL lags of the same count, for comparison
     pure = table[sel].copy()
     pure[:, 4:8] = table[0, 4:8] * 0 + np.array([np.cos(np.deg2rad(3.0)), -np.sin(np.deg2rad(3.0)),
                                                np.sin(np.deg2rad(3.0)), np.cos(np.deg2rad(3.0))])
     pure[:, 2:4] = table[0, 2:4] * 0 + a.hdr_small["CDELT1"] / 3600.0
-    eng.flags = _ext.make_flags(False, 1)
+    eng.flags |= _ext.FLAG_PURE_SHIFT
     tab = eng._upload(pure)
     out = torch.empty(n, dtype=torch.float64, device=eng.device)
     eng.evaluate(tab, out)

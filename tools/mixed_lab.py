@@ -22,7 +22,8 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--steps", type=int, default=3)
     ap.add_argument("--out", default="gpurun_out/mixed_lab.json")
-    ap.add_argument("--combos", default="fp64:0,mixed:0,mixed:1,mixed:3,mixed:4")
+    ap.add_argument("--combos", default="fp64:0,mixed:0,mixed:1",
+                    help="arithmetic:variant pairs; variant 0 = flavour from the lag grid, 1 = pure-shift flavour")
     ap.add_argument("--lagsets", default="config1,rotated")
     args = ap.parse_args()
     pl, ps = bench.ensure_config1()

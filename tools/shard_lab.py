@@ -1,5 +1,5 @@
 """Per-shard cost of the config-1 search: K1 time of each of the G contiguous lag slices on one GPU (GPU box).
-    COREG_WAVES=64 python tools/shard_lab.py --shards 8
+    python tools/shard_lab.py --shards 8
 Tells a load imbalance between ranks (slices differ) from a per-launch overhead (all slices above total / G)."""
 import argparse
 import json
@@ -55,7 +55,7 @@ def main():
         ms, k = _ext.profile_end()
         out.append({"shard": r, "lags": int(len(sel)), "k1_ms": ms / args.steps, "us_per_lag": 1e3 * ms / args.steps / len(sel)})
         print(json.dumps(out[-1]), flush=True)
-    print(json.dumps({"waves": os.environ.get("COREG_WAVES", "128"), "interleave": args.interleave,
+    print(json.dumps({"interleave": args.interleave,
                       "max_shard_ms": max(o["k1_ms"] for o in out[1:]), "mean_shard_ms": float(np.mean([o["k1_ms"] for o in out[1:]])),
                       "whole_over_G_ms": out[0]["k1_ms"] / args.shards}))
 
