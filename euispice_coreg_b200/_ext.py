@@ -46,6 +46,14 @@ class CoregSurfaceFrames(C.Structure):
                                           "dt_days", "rsun")]
 
 
+class CoregRegions(C.Structure):
+    _fields_ = [("block_h", C.c_int), ("block_w", C.c_int), ("ld", C.c_int64), ("corr_dev", C.c_void_p),
+                ("nvalid_dev", C.c_void_p)]
+
+
+REGION_ALIGN = 64   # block sides of the per-block outputs: multiples of the lag kernels' 64-pixel tile sides
+
+
 LAG_TAN_DOUBLES = 10    # sizeof(CoregLagTan) / 8
 LAG_TAN_EDGE_DOUBLES = 12   # sizeof(CoregLagTanEdge) / 8
 TAN_WCS_DOUBLES = 11    # sizeof(CoregTanWcs) / 8
@@ -85,6 +93,12 @@ _SIGNATURES = {
                                      C.c_int, _P, _P, C.c_size_t, _P, _P, C.c_int, _P]),
     "coreg_hpc_lag_corr_wcs": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(CoregTanWcs),
                                          _P, C.c_int64, C.c_int, _P, _P, C.c_size_t, _P, _P, C.c_int, _P]),
+    "coreg_hpc_lag_corr_regions": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int64,
+                                             C.c_int, _P, _P, C.c_size_t, _P, _P, C.POINTER(CoregRegions), C.c_int,
+                                             _P]),
+    "coreg_hpc_lag_corr_wcs_regions": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(CoregTanWcs),
+                                                 _P, C.c_int64, C.c_int, _P, _P, C.c_size_t, _P, _P,
+                                                 C.POINTER(CoregRegions), C.c_int, _P]),
     "coreg_hpc_lag_corr_wcs_mixed": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int,
                                                C.POINTER(CoregTanWcs), _P, C.c_int64, C.c_int, _P, _P, C.c_size_t, _P,
                                                _P, _P, C.c_int, _P]),
@@ -395,8 +409,32 @@ def lag_corr_workspace_bytes(gnx, gny, n_lags, offset_window=False):
     return int(fn(int(gnx), int(gny), int(n_lags)))
 
 
-def hpc_lag_corr(ref, small, planes, lags, order, pivots, work, corr_out, nvalid_out=None, flags=0):
-    """K1. `lags`: device float64 [n_lags, 10] (CoregLagTan rows). Writes corr_out[n_lags]."""
+def region_grid(gny, gnx, block_h, block_w):
+    """(nby, nbx): blocks of block_h x block_w pixels over a gny x gnx grid from pixel (0, 0), the last block row and
+    column clipped to the grid (`CoregRegions`)."""
+    return -(-int(gny) // int(block_h)), -(-int(gnx) // int(block_w))
+
+
+def _regions_struct(regions, gny, gnx, n_lags):
+    """regions = (block_h, block_w, corr [n_blocks, >= n_lags] float64, nvalid [n_blocks, >= n_lags] int64) ->
+    `CoregRegions`. The outputs may be column slices [:, lo:hi] of wider device arrays: ld is their row stride."""
+    torch = _torch()
+    bh, bw, corr, nvalid = regions
+    if not (corr.is_cuda and nvalid.is_cuda):
+        raise CoregLibraryError("device tensors expected for the per-block outputs")
+    if corr.dtype != torch.float64 or nvalid.dtype != torch.int64:
+        raise TypeError("per-block outputs: float64 corr and int64 nvalid")
+    if corr.dim() != 2 or corr.shape != nvalid.shape or corr.stride() != nvalid.stride() or \
+            (corr.shape[1] > 1 and corr.stride(1) != 1) or corr.shape[1] < n_lags:
+        raise ValueError("per-block outputs: two [n_blocks, >= n_lags] arrays with unit column stride and equal strides")
+    if bh > 0 and bw > 0 and corr.shape[0] != int(np.prod(region_grid(gny, gnx, bh, bw))):
+        raise ValueError("per-block outputs: one row per block of the grid")
+    return CoregRegions(int(bh), int(bw), corr.stride(0), corr.data_ptr(), nvalid.data_ptr())
+
+
+def hpc_lag_corr(ref, small, planes, lags, order, pivots, work, corr_out, nvalid_out=None, flags=0, regions=None):
+    """K1. `lags`: device float64 [n_lags, 10] (CoregLagTan rows). Writes corr_out[n_lags]. `regions` =
+    (block_h, block_w, corr_blocks, nvalid_blocks): also the per-block outputs (`coreg_hpc_lag_corr_regions`)."""
     torch = _torch()
     lib = load()
     _require_cuda(ref, small, planes, lags, pivots, work, corr_out)
@@ -404,12 +442,16 @@ def hpc_lag_corr(ref, small, planes, lags, order, pivots, work, corr_out, nvalid
         raise TypeError("ref must be float32 (the reference keeps the cut large image in float32)")
     n_lags = lags.shape[0]
     gny, gnx = ref.shape
+    args = (_ptr(ref), _ptr(small), _dt(small), small.shape[1], small.shape[0], gnx, gny, _ptr(planes), _ptr(lags),
+            n_lags, int(order), _ptr(pivots), _ptr(work), work.numel() * work.element_size(), _ptr(corr_out),
+            _ptr(nvalid_out) if nvalid_out is not None else None)
     with torch.cuda.device(ref.device):
-        _check(lib.coreg_hpc_lag_corr(_ptr(ref), _ptr(small), _dt(small), small.shape[1], small.shape[0], gnx, gny,
-                                      _ptr(planes), _ptr(lags), n_lags, int(order), _ptr(pivots), _ptr(work),
-                                      work.numel() * work.element_size(), _ptr(corr_out),
-                                      _ptr(nvalid_out) if nvalid_out is not None else None,
-                                      int(flags), _stream()), "coreg_hpc_lag_corr")
+        if regions is not None:
+            rg = _regions_struct(regions, gny, gnx, n_lags)
+            _check(lib.coreg_hpc_lag_corr_regions(*args, C.byref(rg), int(flags), _stream()),
+                   "coreg_hpc_lag_corr_regions")
+            return
+        _check(lib.coreg_hpc_lag_corr(*args, int(flags), _stream()), "coreg_hpc_lag_corr")
 
 
 def pad_edge(img):
@@ -462,12 +504,13 @@ def hpc_lag_corr_edge(ref, small_pad, planes, lags, pivots, work, corr_out, nval
 
 
 def hpc_lag_corr_wcs(ref, small, grid_wcs, lag_wcs, order, pivots, work, corr_out, nvalid_out=None, flags=0,
-                     small32c=None, flagged=None):
+                     small32c=None, flagged=None, regions=None):
     """K1, homography form. `lag_wcs`: device float64 [n_lags, 11] (CoregTanWcs rows of the shifted headers);
     `grid_wcs`: `_compat.wcs.TanWcs` of the common grid. `small32c` (the float32 payload `small` was widened from,
     centred on its float32 pivot: `center_f32`) selects the mixed-arithmetic kernel -- FP64 projection, FP32 spline --;
     `pivots` must then be the [4, 2] statistics block and `flagged` a zeroed int32 device counter that receives the
-    number of lags tripping the kernel's error-model guard."""
+    number of lags tripping the kernel's error-model guard. `regions` = (block_h, block_w, corr_blocks, nvalid_blocks):
+    also the per-block outputs (`coreg_hpc_lag_corr_wcs_regions`; not with mixed arithmetic)."""
     torch = _torch()
     lib = load()
     _require_cuda(ref, small, lag_wcs, pivots, work, corr_out)
@@ -477,6 +520,17 @@ def hpc_lag_corr_wcs(ref, small, grid_wcs, lag_wcs, order, pivots, work, corr_ou
         raise TypeError("the homography kernel reads a float64 small image")
     gny, gnx = ref.shape
     g = tan_struct(grid_wcs)
+    if regions is not None:
+        if small32c is not None:
+            raise ValueError("no per-block outputs in mixed arithmetic (its guard is calibrated on whole-grid moments)")
+        rg = _regions_struct(regions, gny, gnx, lag_wcs.shape[0])
+        with torch.cuda.device(ref.device):
+            _check(lib.coreg_hpc_lag_corr_wcs_regions(
+                _ptr(ref), _ptr(small), small.shape[1], small.shape[0], gnx, gny, C.byref(g), _ptr(lag_wcs),
+                lag_wcs.shape[0], int(order), _ptr(pivots), _ptr(work), work.numel() * work.element_size(),
+                _ptr(corr_out), _ptr(nvalid_out) if nvalid_out is not None else None, C.byref(rg), int(flags),
+                _stream()), "coreg_hpc_lag_corr_wcs_regions")
+        return
     if small32c is not None:
         _require_cuda(small32c, flagged)
         if small32c.dtype != torch.float32 or small32c.shape != small.shape:

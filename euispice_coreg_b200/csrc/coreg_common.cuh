@@ -264,6 +264,52 @@ inline RollWLayout rollw_layout(int gnx, int gny, int64_t n_lags) {
   L.total = L.mask + ((tiles * (size_t)n_lags * sizeof(unsigned) + 15) / 16) * 16;
   return L;
 }
+// ---- per-block outputs of the lag search (CoregRegions) ----
+// Block sides are multiples of 64 grid pixels, so every block edge is a tile edge of both lag kernels (64 x 64 rolling,
+// 64 x 16 generic) and a block's moments are the sum of whole tiles' records. Refused before any CUDA call: a bad
+// block side, ld < n_lags, more blocks than one launch can index, and COREG_FLAG_MIXED (the mixed kernel's per-lag
+// guard is calibrated on whole-grid moments).
+constexpr int kRegionAlign = 64;
+inline int check_regions(const CoregRegions* rg, int gnx, int gny, int64_t n_lags, int flags, const char* entry) {
+  if (!rg || !rg->corr_dev || !rg->nvalid_dev) return fail(COREG_EINVAL, "%s: null CoregRegions pointer", entry);
+  if (rg->block_h <= 0 || rg->block_w <= 0 || rg->block_h % kRegionAlign || rg->block_w % kRegionAlign)
+    return fail(COREG_EINVAL, "%s: block sides must be positive multiples of 64 pixels", entry);
+  if (rg->ld < n_lags) return fail(COREG_EINVAL, "%s: CoregRegions.ld < n_lags", entry);
+  if (flags & COREG_FLAG_MIXED) return fail(COREG_EINVAL, "%s: no per-block outputs in mixed arithmetic", entry);
+  if (gnx > 0 && gny > 0 &&
+      (int64_t)((gny + rg->block_h - 1) / rg->block_h) * ((gnx + rg->block_w - 1) / rg->block_w) > 65535)
+    return fail(COREG_EINVAL, "%s: more than 65535 blocks", entry);
+  return COREG_OK;
+}
+
+// Pearson r of a fold of moments (NaN without a valid pixel): the arithmetic of the whole-grid finalize kernels
+__device__ __forceinline__ double pearson_from_moments(double n, double sa, double sb, double saa, double sbb,
+                                                       double sab) {
+  double r = CUDART_NAN;
+  if (n > 0.0) {
+    const double cov = sab - sa * sb / n;
+    const double va = saa - sa * sa / n;
+    const double vb = sbb - sb * sb / n;
+    r = cov / sqrt(va * vb);
+  }
+  return r;
+}
+
+// tiles [ty0, ty1) x [tx0, tx1) of block `blk` (row-major over nbx blocks per row; bt_h x bt_w tiles per block, the
+// last block row / column clipped to the grid)
+struct RegionTiles {
+  int ty0, tx0, ntx, n_tiles;
+};
+__device__ __forceinline__ RegionTiles region_tiles(int blk, int nbx, int bt_h, int bt_w, int tiles_x, int tiles_y) {
+  RegionTiles R;
+  const int by = blk / nbx, bx = blk - by * nbx;
+  R.ty0 = by * bt_h;
+  R.tx0 = bx * bt_w;
+  R.ntx = min(tiles_x, R.tx0 + bt_w) - R.tx0;
+  R.n_tiles = (min(tiles_y, R.ty0 + bt_h) - R.ty0) * R.ntx;
+  return R;
+}
+
 inline size_t partials_bytes(int gnx, int gny, int64_t n_lags) {
   const size_t tiles = (size_t)((gnx + kTileW - 1) / kTileW) * ((gny + kMinTileH - 1) / kMinTileH);
   // a multiple of 16: the per-lag homographies (16-byte aligned records) follow the partials in the workspace
@@ -469,8 +515,7 @@ struct HomLag {
 
 // ---- launchers defined in one translation unit and used from another ----
 // fixed-order fold of [tile][lag][kMom] partials -> Pearson r (coreg_lag_generic.cu)
-int launch_finalize_tiles(const double* work, int tiles, int64_t n_lags, double* corr, int64_t* nvalid, cudaStream_t s);
-// Carrington-frame lag kernel + its finalize (coreg_lag_offset.cu); small_dtype COREG_F32 / COREG_F64
+int launch_finalize_tiles(const double* work, int tiles, int64_t n_lags, double* corr, int64_t* nvalid, cudaStream_t s);// Carrington-frame lag kernel + its finalize (coreg_lag_offset.cu); small_dtype COREG_F32 / COREG_F64
 int launch_offset_fast(int gnx, int gny, int64_t n_lags, cudaStream_t s, const double* ref, const void* small,
                        int small_dtype, int snx, int sny, const double* tx, const double* ty,
                        const CoregLagOffset* lags, const double* pivots, void* work, double* corr, int64_t* nvalid);

@@ -156,6 +156,52 @@ int launch_finalize_tiles(const double* work, int tiles, int64_t n_lags, double*
   return COREG_OK;
 }
 
+// Per-block form of lag_corr_finalize_kernel (CoregRegions): blockIdx.y = block of the grid. The block's tiles are taken
+// in ascending order and its k-th tile goes to thread k % 128, as the whole-grid fold deals tile k: one block covering
+// the grid folds the same sums in the same order.
+__global__ void __launch_bounds__(128)
+lag_corr_finalize_regions_kernel(const double* __restrict__ work, int n_lags, int tiles_x, int tiles_y, int bt_h,
+                                 int bt_w, int nbx, double* __restrict__ corr, int64_t* __restrict__ nvalid,
+                                 int64_t ld) {
+  __shared__ double s[128][6];
+  const RegionTiles R = region_tiles(blockIdx.y, nbx, bt_h, bt_w, tiles_x, tiles_y);
+  const int lag = blockIdx.x;
+  double m[6] = {0, 0, 0, 0, 0, 0};
+  for (int k = threadIdx.x; k < R.n_tiles; k += 128) {
+    const int t = (R.ty0 + k / R.ntx) * tiles_x + R.tx0 + k % R.ntx;
+    const double* p = work + ((size_t)t * n_lags + lag) * kMom;
+#pragma unroll
+    for (int q = 0; q < 6; ++q) m[q] += p[q];
+  }
+#pragma unroll
+  for (int q = 0; q < 6; ++q) s[threadIdx.x][q] = m[q];
+  __syncthreads();
+  for (int o = 64; o > 0; o >>= 1) {
+    if (threadIdx.x < o) {
+#pragma unroll
+      for (int q = 0; q < 6; ++q) s[threadIdx.x][q] += s[threadIdx.x + o][q];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    const size_t o = (size_t)blockIdx.y * ld + lag;
+    corr[o] = pearson_from_moments(s[0][0], s[0][1], s[0][2], s[0][3], s[0][4], s[0][5]);
+    nvalid[o] = (int64_t)s[0][0];
+  }
+}
+
+// the per-block fold of the tile partials a launch_lag call left in `work` (tiles of 64 x kMinTileH pixels)
+int launch_finalize_tiles_regions(const double* work, int gnx, int gny, int64_t n_lags, const CoregRegions* rg,
+                                  cudaStream_t s) {
+  const int tiles_x = (gnx + kTileW - 1) / kTileW, tiles_y = (gny + kMinTileH - 1) / kMinTileH;
+  const int nbx = (gnx + rg->block_w - 1) / rg->block_w, nby = (gny + rg->block_h - 1) / rg->block_h;
+  lag_corr_finalize_regions_kernel<<<dim3((unsigned)n_lags, (unsigned)(nbx * nby)), 128, 0, s>>>(
+      work, (int)n_lags, tiles_x, tiles_y, rg->block_h / kMinTileH, rg->block_w / kTileW, nbx, rg->corr_dev,
+      rg->nvalid_dev, rg->ld);
+  CK_LAUNCH("lag_corr_finalize_regions_kernel");
+  return COREG_OK;
+}
+
 // generic kernel: 4 pixels per thread, 4 CTAs / SM. (Measured and dropped: 8 pixels per thread at 2 CTAs / SM,
 // 115.7 vs 101.9 ms on 2048 x 1024 Carrington maps with 3600 lags, profiles/r1_widened_kernels.md.)
 template <class Coord, int ORDER, bool STRICT, typename SmallT, typename RefT, bool ROUND32>
@@ -259,6 +305,18 @@ int coreg_hpc_lag_corr(const float* ref, const void* small, int small_dtype, int
                                                          n_lags, order, pivots, work, work_bytes, corr, nvalid, flags,
                                                          s);
   return fail(COREG_EINVAL, "small_dtype must be COREG_F32 or COREG_F64");
+}
+
+int coreg_hpc_lag_corr_regions(const float* ref, const void* small, int small_dtype, int snx, int sny, int gnx, int gny,
+                               const double* planes, const CoregLagTan* lags, int64_t n_lags, int order,
+                               const double* pivots, void* work, size_t work_bytes, double* corr, int64_t* nvalid,
+                               const CoregRegions* regions, int flags, void* stream) {
+  if (int rc = check_regions(regions, gnx, gny, n_lags, flags, "coreg_hpc_lag_corr_regions")) return rc;
+  int rc = coreg_hpc_lag_corr(ref, small, small_dtype, snx, sny, gnx, gny, planes, lags, n_lags, order, pivots, work,
+                              work_bytes, corr, nvalid, flags, stream);
+  if (rc || n_lags <= 0) return rc;
+  return launch_finalize_tiles_regions(static_cast<const double*>(work), gnx, gny, n_lags, regions,
+                                       (cudaStream_t)stream);
 }
 
 int coreg_hpc_lag_corr_edge(const double* ref, const double* small_pad, int snx, int sny, int gnx, int gny,

@@ -901,6 +901,7 @@ lag_corr_roll_kernel(const RefT* __restrict__ ref, const double* __restrict__ sm
 // compared with the sampled image's own variance and flagged[lag] = 1 marks the lags that cannot be trusted to 1e-7
 // (the caller re-evaluates those with the all-FP64 kernel).
 constexpr int kFinGroups = 10, kFinElems = kRollChunk * 3;
+constexpr int kRollRows = 16;   // rows per thread of the launched rolling kernel: tiles of 64 x 64 grid pixels
 
 __device__ __forceinline__ bool mixed_guard_trips(const double* __restrict__ guard, double n, double vb) {
   // guard = [4][2] statistics block: row 2 = max |v|, row 3 = RMS of (v - pivot); column 1 = the small image.
@@ -973,6 +974,74 @@ lag_corr_finalize_w_kernel(const double* __restrict__ wrec, const double* __rest
   }
 }
 
+// Per-block form of lag_corr_finalize_w_kernel (CoregRegions): blockIdx.y = block of the grid. The block's record rows
+// are taken in ascending order (tile rows, tiles, warps) and its k-th row goes to row group k % kFinGroups, as the
+// whole-grid fold deals row k: one block covering the grid folds the same sums in the same order.
+__global__ void __launch_bounds__(256)
+lag_corr_finalize_w_regions_kernel(const double* __restrict__ wrec, const double* __restrict__ wcorr,
+                                   const double* __restrict__ wconst, const unsigned* __restrict__ wmask, int n_lags,
+                                   int tiles_x, int tiles_y, int bt_h, int bt_w, int nbx, double* __restrict__ corr,
+                                   int64_t* __restrict__ nvalid, int64_t ld) {
+  __shared__ double s_var[kFinGroups][kFinElems], s_cst[kFinGroups][kFinElems];
+  __shared__ double s_tot[2][kFinElems];
+  const RegionTiles R = region_tiles(blockIdx.y, nbx, bt_h, bt_w, tiles_x, tiles_y);
+  const int n_rows = R.n_tiles * kWarps;
+  const int l0 = blockIdx.x * kRollChunk;
+  const int t = threadIdx.x, e = t % kFinElems, g = t / kFinElems;
+  const int lag = l0 + e / 3, v = e % 3;
+  if (g < kFinGroups) {
+    double av = 0.0, ac = 0.0;
+    if (lag < n_lags) {
+      for (int k = g; k < n_rows; k += kFinGroups) {
+        const int tl = k / kWarps;
+        const int tile = (R.ty0 + tl / R.ntx) * tiles_x + R.tx0 + tl % R.ntx;
+        const size_t r = (size_t)tile * kWarps + k % kWarps;
+        const size_t o = (r * n_lags + lag) * 3 + v;
+        av += wrec[o];
+        ac += wconst[r * 3 + v];
+        if ((wmask[(size_t)tile * n_lags + lag] >> (k % kWarps)) & 1u) ac -= wcorr[o];
+      }
+    }
+    s_var[g][e] = av;
+    s_cst[g][e] = ac;
+  }
+  __syncthreads();
+  if (t < kFinElems) {
+    double av = s_var[0][t], ac = s_cst[0][t];
+#pragma unroll
+    for (int k = 1; k < kFinGroups; ++k) {
+      av += s_var[k][t];
+      ac += s_cst[k][t];
+    }
+    s_tot[0][t] = av;
+    s_tot[1][t] = ac;
+  }
+  __syncthreads();
+  if (t < kRollChunk && l0 + t < n_lags) {
+    const double n = s_tot[1][3 * t];
+    const size_t o = (size_t)blockIdx.y * ld + l0 + t;
+    corr[o] = pearson_from_moments(n, s_tot[1][3 * t + 1], s_tot[0][3 * t], s_tot[1][3 * t + 2], s_tot[0][3 * t + 1],
+                                   s_tot[0][3 * t + 2]);
+    nvalid[o] = (int64_t)n;
+  }
+}
+
+// the per-block fold of the records a launch_lag_rollw call left in `work` (its tiles: kRollRows rows per thread)
+int launch_finalize_w_regions(int gnx, int gny, int64_t n_lags, void* work, const CoregRegions* rg, cudaStream_t s) {
+  constexpr int TILE_H = kRowsPerPass * kRollRows;
+  const RollWLayout L = rollw_layout(gnx, gny, n_lags);
+  char* base = static_cast<char*>(work);
+  const int tiles_x = (gnx + kTileW - 1) / kTileW, tiles_y = (gny + TILE_H - 1) / TILE_H;
+  const int nbx = (gnx + rg->block_w - 1) / rg->block_w, nby = (gny + rg->block_h - 1) / rg->block_h;
+  const dim3 grid((unsigned)((n_lags + kRollChunk - 1) / kRollChunk), (unsigned)(nbx * nby));
+  lag_corr_finalize_w_regions_kernel<<<grid, 256, 0, s>>>(
+      reinterpret_cast<const double*>(base + L.rec), reinterpret_cast<const double*>(base + L.corr),
+      reinterpret_cast<const double*>(base + L.cst), reinterpret_cast<const unsigned*>(base + L.mask), (int)n_lags,
+      tiles_x, tiles_y, rg->block_h / TILE_H, rg->block_w / kTileW, nbx, rg->corr_dev, rg->nvalid_dev, rg->ld);
+  CK_LAUNCH("lag_corr_finalize_w_regions_kernel");
+  return COREG_OK;
+}
+
 // rolling kernel + its finalize: 16 rows per thread, 2 CTAs / SM. `adapt` selects the flavour with the adaptive segment
 // for rotated / rescaled lags; without it (COREG_FLAG_PURE_SHIFT) the kernel serves lag grids of pure CRVAL shifts,
 // where no segment drifts. The adaptive code is never executed there, but its presence in the kernel costs the regular
@@ -989,7 +1058,7 @@ int launch_lag_rollw(bool adapt, int gnx, int gny, int64_t n_lags, int sms, cuda
                      const double* small, const float* small32, int snx, int sny,
                      const HomLag* ft, const double* pivots, void* work, double* corr, int64_t* nvalid, bool prof,
                      int* flagged) {
-  constexpr int P = 16, MINB = 2;
+  constexpr int P = kRollRows, MINB = 2;
   const bool mixed = small32 != nullptr;
   const RollWLayout L = rollw_layout(gnx, gny, n_lags);
   char* base = static_cast<char*>(work);
@@ -1066,6 +1135,17 @@ int coreg_hpc_lag_corr_wcs(const float* ref, const double* small, int snx, int s
   if (work_bytes < coreg_lag_corr_workspace_bytes(gnx, gny, n_lags)) return fail(COREG_ENOMEM, "workspace too small");
   return hpc_lag_corr_wcs_impl(ref, small, nullptr, snx, sny, gnx, gny, grid_wcs, lag_wcs, n_lags, pivots, work, corr,
                                nvalid, flags, (cudaStream_t)stream);
+}
+
+int coreg_hpc_lag_corr_wcs_regions(const float* ref, const double* small, int snx, int sny, int gnx, int gny,
+                                   const CoregTanWcs* grid_wcs, const CoregTanWcs* lag_wcs, int64_t n_lags, int order,
+                                   const double* pivots, void* work, size_t work_bytes, double* corr, int64_t* nvalid,
+                                   const CoregRegions* regions, int flags, void* stream) {
+  if (int rc = check_regions(regions, gnx, gny, n_lags, flags, "coreg_hpc_lag_corr_wcs_regions")) return rc;
+  int rc = coreg_hpc_lag_corr_wcs(ref, small, snx, sny, gnx, gny, grid_wcs, lag_wcs, n_lags, order, pivots, work,
+                                  work_bytes, corr, nvalid, flags, stream);
+  if (rc || n_lags <= 0) return rc;
+  return launch_finalize_w_regions(gnx, gny, n_lags, work, regions, (cudaStream_t)stream);
 }
 
 int coreg_hpc_lag_corr_wcs_mixed(const float* ref, const double* small, const float* small32c, int snx, int sny,

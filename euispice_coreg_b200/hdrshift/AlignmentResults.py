@@ -163,3 +163,32 @@ class AlignmentResults:
                 f"\n dy = {s[3]} '' \n dcrot = {s[4]} deg")
 
     __repr__ = __str__
+
+
+class LocalAlignmentResults:
+    """Per-block correlation cubes of one helioprojective search (`Alignment(..., local_block=...)`): the common grid
+    cut into blocks from pixel (0, 0), the last block row and column taking whatever remains.
+
+    corr       [nby, nbx, n_crval1, n_crval2, n_cdelt1, n_cdelt2, n_crota, n_solar_r] float64: Pearson r of each block's
+               pixels; NaN where a block has no valid pixel pair under a lag, 0.0 for lags the reference cannot
+               evaluate (as in the global cube)
+    nvalid     [nby, nbx, n_crval1, ..., n_crota] int64: valid pixel pairs per block and lag (they sum to the global count)
+    bounds     [nby, nbx, 4] int64: (row0, row1, col0, col1) of each block on the common grid
+    max_index  [nby, nbx, 6] int64: the cube index of each block's maximum (first occurrence, C order, NaN ignored), -1
+               for a block that is NaN at every lag
+    """
+
+    def __init__(self, corr, nvalid, bounds, **results_kwargs):
+        self.corr = corr
+        self.nvalid = nvalid
+        self.bounds = bounds
+        self.max_index = np.full(corr.shape[:2] + (corr.ndim - 2,), -1, dtype=np.int64)
+        flat = corr.reshape(corr.shape[:2] + (-1,))
+        some = ~np.isnan(flat).all(axis=-1)
+        if some.any():
+            self.max_index[some] = np.stack(np.unravel_index(np.nanargmax(flat[some], axis=-1), corr.shape[2:]), -1)
+        self._results_kwargs = results_kwargs
+
+    def results(self, i, j):
+        """`AlignmentResults` of block (i, j): its arg-max and Gaussian sub-lag fit, as for the whole grid."""
+        return AlignmentResults(corr=self.corr[i, j], **self._results_kwargs)

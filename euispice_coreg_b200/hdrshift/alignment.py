@@ -13,6 +13,7 @@ that kill the reference's worker, App. B1) are reported as 0.0 exactly like the 
 from __future__ import annotations
 
 import copy
+import os
 import warnings
 
 import numpy as np
@@ -21,7 +22,7 @@ from .._compat import fits_lite, units
 from .._compat.wcs import CarWcs, TanWcs
 from ..utils import Util
 from . import engine as _engine
-from .AlignmentResults import AlignmentResults
+from .AlignmentResults import AlignmentResults, LocalAlignmentResults
 
 
 def _open_fits(path):
@@ -43,7 +44,7 @@ class Alignment:
                  small_fov_window: object = -1,
                  path_save_figure: str = None, reprojection_order=2, force_crota_0=False,
                  unit_lag="arcsec", cdelt_semantics="reference", strict_arithmetic=False, lag_search="dense",
-                 coarse_stride=None, arithmetic=None):
+                 coarse_stride=None, arithmetic=None, local_block=None):
         """Same parameters as the reference (`hdrshift/alignment.py:47-83`). Additions:
 
         arithmetic: "fp64" (default): every sample is evaluated in FP64 like the reference does (scipy accumulates in
@@ -65,6 +66,14 @@ class Alignment:
             window's edge; lags that were not evaluated are NaN in the cube. Every evaluated entry is bit-identical
             to the dense cube's; the arg-max is the dense one whenever the correlation peak is wider than the
             stride (default stride: the large image's pixel size in lag steps, at least 2).
+        local_block: None (default) or the block size (rows, cols) -- or one int for square blocks -- in pixels of the
+            common grid, each a positive multiple of 64. `align_using_helioprojective` then also returns, from the same
+            pass of the lag kernels, one correlation cube per block of the common grid (blocks from pixel (0, 0), the
+            last block row and column taking whatever remains): `.local`, a `LocalAlignmentResults`, on this object and
+            on the returned `AlignmentResults`. A shift that changes across the field (pointing drift along a SPICE
+            raster, a roll or plate-scale error) shows up as block maxima that differ. Not with
+            lag_search="coarse_to_fine" (its windows follow the global maximum), mixed arithmetic, or the Carrington
+            entry points.
         """
         self.large_fov_known_pointing = large_fov_known_pointing
         self.small_fov_to_correct = small_fov_to_correct
@@ -114,6 +123,15 @@ class Alignment:
             raise ValueError("lag_search must be 'dense' or 'coarse_to_fine'")
         self.lag_search = lag_search
         self.coarse_stride = coarse_stride
+        self.local_block = None if local_block is None else _engine.local_block_shape(local_block)
+        self.local = None
+        if self.local_block is not None:
+            if lag_search != "dense":
+                raise ValueError("local_block needs lag_search='dense' (the coarse-to-fine windows follow the global "
+                                 "maximum)")
+            if arithmetic == "mixed":
+                raise ValueError("local_block needs all-FP64 arithmetic (the mixed kernel's per-lag guard is "
+                                 "calibrated on whole-grid moments)")
         self.lags_evaluated = None
         self.engine = None
         self.nvalid = None
@@ -149,6 +167,7 @@ class Alignment:
         "fa" (`_carrington_transform_fa`, the default) or "sunpy" (`_carrington_transform_sunpy`, `:939-985`: no grid
         arguments needed; the search runs on the small image's own grid after a solar-surface reprojection of the large
         image -- a restatement of sunpy / reproject's published algorithm, `_surface_search`)."""
+        self._refuse_local_block("align_using_carrington")
         self.method = method
         self.coordinate_frame = "final_carrington"
         self.lon_ctype = "HPLN-TAN"
@@ -193,6 +212,7 @@ class Alignment:
         rounded to float32 when read (`:373, 387`), lags converted to header units without longitude wrapping
         (`:388, 831-837`), and -- unlike the other two entry points -- the lag arrays handed to `AlignmentResults`
         as they are (`:392-399`)."""
+        self._refuse_local_block("align_using_initial_carrington")
         self.lonlims = None
         self.latlims = None
         self.shape = None
@@ -223,6 +243,10 @@ class Alignment:
                                     reference_image_path=self.large_fov_known_pointing,
                                     reference_image_window=self.large_fov_window)
         return results
+
+    def _refuse_local_block(self, entry):
+        if getattr(self, "local_block", None) is not None:
+            raise ValueError(f"local_block is implemented for align_using_helioprojective only, not {entry}")
 
     # ------------------------------------------------------------------------------------------------
     # host preparation (mirrors alignment.py:299-316, 580-611, 799-887)
@@ -268,6 +292,7 @@ class Alignment:
 
     def _wrap_results(self, results, return_type):
         if return_type == "corr":
+            self._wrap_local()
             return results
         if return_type == "AlignmentResults":
             conv = lambda v: units.convert(units.ang2pipi(v, self.unit_lag), self.unit_lag, self.unit_lag_input)  # noqa: E731
@@ -276,13 +301,28 @@ class Alignment:
             self.lag_cdelt1 = conv(self.lag_cdelt1)
             self.lag_cdelt2 = conv(self.lag_cdelt2)
             self.unit_lag = self.unit_lag_input
-            return AlignmentResults(corr=results, lag_crval1=self.lag_crval1, lag_crval2=self.lag_crval2,
-                                    lag_cdelt1=self.lag_cdelt1, lag_cdelt2=self.lag_cdelt2, lag_crota=self.lag_crota,
-                                    unit_lag=self.unit_lag_input, image_to_align_path=self.small_fov_to_correct,
-                                    image_to_align_window=self.small_fov_window,
-                                    reference_image_path=self.large_fov_known_pointing,
-                                    reference_image_window=self.large_fov_window)
+            res = AlignmentResults(corr=results, **self._results_kwargs())
+            if self._wrap_local() is not None:
+                res.local = self.local
+            return res
+        self._wrap_local()
         return results
+
+    def _results_kwargs(self):
+        """Everything but the cube that `AlignmentResults` takes, with the lag arrays as they stand (header units
+        after a search, the caller's units once `_wrap_results` has converted them back)."""
+        return dict(lag_crval1=self.lag_crval1, lag_crval2=self.lag_crval2, lag_cdelt1=self.lag_cdelt1,
+                    lag_cdelt2=self.lag_cdelt2, lag_crota=self.lag_crota, unit_lag=self.unit_lag,
+                    image_to_align_path=self.small_fov_to_correct, image_to_align_window=self.small_fov_window,
+                    reference_image_path=self.large_fov_known_pointing, reference_image_window=self.large_fov_window)
+
+    def _wrap_local(self):
+        """`LocalAlignmentResults` of the per-block cubes the last search left (None without `local_block`)."""
+        raw = getattr(self, "_local_raw", None)
+        if raw is not None:
+            self._local_raw = None
+            self.local = LocalAlignmentResults(*raw, **self._results_kwargs())
+        return getattr(self, "local", None)
 
     def _check_ant_create_pcij_matrix(self, hdr):
         """`alignment.py:580-611`."""
@@ -428,6 +468,10 @@ class Alignment:
         (`alignment.py:613-797`, parallel branch)."""
         if self.method != 'correlation':
             raise NotImplementedError("only method='correlation' is on the device path")
+        self.local = self._local_raw = None
+        if getattr(self, "local_block", None) is not None and \
+                (getattr(self, "arithmetic", None) or os.environ.get("COREG_ARITHMETIC")) == "mixed":
+            raise ValueError("local_block needs all-FP64 arithmetic (COREG_ARITHMETIC=mixed is set)")
         self._set_removed_values_to_nan_in_datasmall(fov_limits=fov_limits, remove_fov_limits=remove_fov_limits)
         self._set_initial_header_values(ang2pipi)
         if self.unit_lag != self.hdr_small["CUNIT1"] or self.unit_lag != self.hdr_small["CUNIT2"]:
@@ -460,6 +504,17 @@ class Alignment:
             table, dead = eng.hpc_lag_table(self.hdr_small, refs, d1, d2, d3, d4, d5, self.cdelt_semantics)
             if self.lag_search == "coarse_to_fine":
                 corr, nvalid = self._coarse_to_fine(eng, table, shape5, w_large, dead)
+            elif getattr(self, "local_block", None) is not None:
+                corr, nvalid, corr_b, nvalid_b = eng.search(table, block=self.local_block)
+                self.lags_evaluated = int(table.shape[0])
+                nb = corr_b.shape[:2]
+                if dead.any():       # dead lags read 0.0 in every block, as in the cube
+                    corr_b = np.where(dead, 0.0, corr_b)
+                cube_b = corr_b.reshape(nb + shape5 + (1,))
+                if n_r > 1:
+                    cube_b = np.repeat(cube_b, n_r, axis=-1)
+                bounds = _engine.region_bounds(eng.ref.shape[0], eng.ref.shape[1], self.local_block)
+                self._local_raw = (cube_b, nvalid_b.reshape(nb + shape5), bounds)
             else:
                 corr, nvalid = eng.search(table, return_nvalid=True)
                 self.lags_evaluated = int(table.shape[0])

@@ -28,15 +28,18 @@ class AlignmentSpice(Alignment):
                  lag_cdelt1=None, lag_cdelt2=None, lag_crota=None, lag_solar_r=None, large_fov_window=-1,
                  small_fov_window=-1, parallelism: bool = False, counts_cpu_max: int = 40,
                  display_progress_bar: bool = False, path_save_figure=None, wavelength_interval_to_sum="all",
-                 sub_fov_window="all"):
+                 sub_fov_window="all", local_block=None):
         """Same parameters as `hdrshift/alignment_spice.py:14-49`. `wavelength_interval_to_sum` is "all" or
         [wave_min, wave_max] in the header's dispersion unit (or astropy quantities); `sub_fov_window` is "all" or
-        [lon_min, lon_max, lat_min, lat_max] in arcsec (or quantities)."""
+        [lon_min, lon_max, lat_min, lat_max] in arcsec (or quantities). `local_block` (rows, cols) or an int, multiples
+        of 64 pixels: per-block cubes as in `Alignment`; (rows >= raster height, 64) gives one cube per band of 64 slit
+        positions, i.e. per stretch of the scan's time."""
         super().__init__(large_fov_known_pointing=large_fov_known_pointing, small_fov_to_correct=small_fov_to_correct,
                          lag_crval1=lag_crval1, lag_crval2=lag_crval2, lag_cdelt1=lag_cdelt1, lag_cdelt2=lag_cdelt2,
                          lag_crota=lag_crota, display_progress_bar=display_progress_bar, lag_solar_r=lag_solar_r,
                          parallelism=parallelism, counts_cpu_max=counts_cpu_max, large_fov_window=large_fov_window,
-                         small_fov_window=small_fov_window, path_save_figure=path_save_figure)
+                         small_fov_window=small_fov_window, path_save_figure=path_save_figure,
+                         local_block=local_block)
         self.sub_fov_window = sub_fov_window
         self.coordinate_frame = None
         self.extend_pixel_size = None

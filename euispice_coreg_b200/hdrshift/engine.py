@@ -186,26 +186,58 @@ def _dist_info():
 
 
 def gather_slices(local, n_total, chunk):
-    """All-gather equal `chunk`-sized slices (last ones padded) into one [n_total] tensor.
+    """All-gather equal `chunk`-sized slices (last ones padded) into one [n_total] tensor; a local [chunk, ...] tensor
+    (e.g. one row of per-block values per lag) gathers into [n_total, ...].
     NCCL: a single `all_gather_into_tensor` (in place: every rank's slice is already at its offset).
     gloo (CPU tests of the host logic): list-based `all_gather`."""
     torch = _torch()
     dist, rank, world = _dist_info()
     if dist is None or world == 1:
         return local[:n_total]
-    full = torch.empty(chunk * world, dtype=local.dtype, device=local.device)
+    rest = tuple(local.shape[1:])
+    full = torch.empty((chunk * world,) + rest, dtype=local.dtype, device=local.device)
     send = local
-    if send.numel() != chunk:
-        pad = torch.full((chunk,), float("nan"), dtype=local.dtype, device=local.device)
-        pad[:send.numel()] = send
+    if send.shape[0] != chunk:
+        pad = torch.full((chunk,) + rest, float("nan"), dtype=local.dtype, device=local.device)
+        pad[:send.shape[0]] = send
         send = pad
     if local.is_cuda:
         dist.all_gather_into_tensor(full, send.contiguous())
     else:
-        parts = [torch.empty(chunk, dtype=local.dtype) for _ in range(world)]
+        parts = [torch.empty((chunk,) + rest, dtype=local.dtype) for _ in range(world)]
         dist.all_gather(parts, send.contiguous())
         full = torch.cat(parts)
     return full[:n_total]
+
+
+def local_block_shape(block):
+    """`local_block` argument -> (rows, cols) of the blocks of the per-block lag search: an int (square blocks) or a
+    pair, each a positive multiple of 64 pixels (`_ext.REGION_ALIGN`: block edges on the lag kernels' tile edges)."""
+    if isinstance(block, (int, np.integer)) and not isinstance(block, bool):
+        block = (block, block)
+    try:
+        rows, cols = block
+    except (TypeError, ValueError):
+        raise ValueError("local_block must be an int or a (rows, cols) pair") from None
+    for v in (rows, cols):
+        if isinstance(v, bool) or not isinstance(v, (int, np.integer)) or v <= 0 or v % _ext.REGION_ALIGN:
+            raise ValueError(f"local_block sides must be positive multiples of {_ext.REGION_ALIGN} pixels, got {block}")
+    return int(rows), int(cols)
+
+
+def region_bounds(gny, gnx, block):
+    """[nby, nbx, 4] int64 pixel rectangles (row0, row1, col0, col1) of the blocks of a gny x gnx common grid: blocks
+    of (rows, cols) pixels from pixel (0, 0), the last block row and column taking whatever remains."""
+    rows, cols = block
+    nby, nbx = _ext.region_grid(gny, gnx, rows, cols)
+    out = np.empty((nby, nbx, 4), dtype=np.int64)
+    y0 = np.arange(nby) * rows
+    x0 = np.arange(nbx) * cols
+    out[..., 0] = y0[:, None]
+    out[..., 1] = np.minimum(y0 + rows, gny)[:, None]
+    out[..., 2] = x0[None, :]
+    out[..., 3] = np.minimum(x0 + cols, gnx)[None, :]
+    return out
 
 
 class LagSearchEngine:
@@ -580,16 +612,21 @@ class LagSearchEngine:
         per_lag = max(1, (_ext.lag_corr_workspace_bytes(gnx, gny, 1025, ow) - fixed) // 1024)
         return max(OFFSET_CHUNK, ((self.max_workspace_bytes - fixed) // per_lag) // OFFSET_CHUNK * OFFSET_CHUNK)
 
-    def evaluate(self, table_dev, out_dev, nvalid_dev=None, planes=None, allow_mixed=True):
+    def evaluate(self, table_dev, out_dev, nvalid_dev=None, planes=None, allow_mixed=True, regions=None):
         """Run the fused kernel over a device lag table [n, k]; results into out_dev[n]. Helioprojective frame:
         k = 11 (`CoregTanWcs` rows, `tan_wcs_table`) selects the homography kernel, k = 10 (`CoregLagTan` rows,
         `tan_lag_table`) the generic one. Asynchronous. With mixed arithmetic `self.lag_flags` receives the per-lag
-        guard verdicts: follow with `resolve_flags` (which synchronises) before trusting `out_dev`."""
+        guard verdicts: follow with `resolve_flags` (which synchronises) before trusting `out_dev`.
+        regions = (rows, cols, corr_blocks [n_blocks, n] float64, nvalid_blocks [n_blocks, n] int64) device arrays
+        (helioprojective frame, all-FP64 arithmetic): also the per-block outputs of every lag, launch slice [lo, hi)
+        into columns [lo, hi)."""
         torch = _torch()
         n = table_dev.shape[0]
         gny, gnx = self.ref.shape
         step = self.lags_per_launch(gnx, gny)
         self.last_launches = 0
+        if regions is not None and (self.frame != "hpc" or self.arithmetic == "mixed"):
+            raise ValueError("per-block outputs: helioprojective frame with all-FP64 arithmetic only")
         mixed = (allow_mixed and self.frame == "hpc" and table_dev.shape[1] == _ext.TAN_WCS_DOUBLES
                  and self._mixed_applies())
         with torch.cuda.device(self.device):
@@ -598,6 +635,7 @@ class LagSearchEngine:
             for lo in range(0, n, step):
                 hi = min(n, lo + step)
                 nv = None if nvalid_dev is None else nvalid_dev[lo:hi]
+                rg = None if regions is None else regions[:2] + (regions[2][:, lo:hi], regions[3][:, lo:hi])
                 if self.frame == "hpc" and table_dev.shape[1] == _ext.TAN_WCS_DOUBLES:
                     flags = self.flags
                     if self.pure_shift_hint:
@@ -607,7 +645,7 @@ class LagSearchEngine:
                     _ext.hpc_lag_corr_wcs(self.ref, self.small, self.grid_wcs, table_dev[lo:hi], self.order,
                                           self.stats if mixed else self.pivots, work, out_dev[lo:hi], nv, flags,
                                           small32c=self.small32 if mixed else None,
-                                          flagged=self.lag_flags[lo:hi] if mixed else None)
+                                          flagged=self.lag_flags[lo:hi] if mixed else None, regions=rg)
                 elif self.frame == "surface":
                     _ext.hpc_lag_corr_edge(self.ref, self.small_pad, self.planes, table_dev[lo:hi], self.pivots, work,
                                            out_dev[lo:hi], nv, self.flags)
@@ -616,12 +654,12 @@ class LagSearchEngine:
                                       self.pivots, work, out_dev[lo:hi], nv, self.flags)
                 elif self.frame == "hpc":
                     _ext.hpc_lag_corr(self.ref, self.small, self._hpc_planes(), table_dev[lo:hi], self.order,
-                                      self.pivots, work, out_dev[lo:hi], nv, self.flags)
+                                      self.pivots, work, out_dev[lo:hi], nv, self.flags, regions=rg)
                 else:
                     tx, ty = planes
                     _ext.offset_lag_corr(self.ref, self.small, tx, ty, table_dev[lo:hi], self.order, self.pivots,
                                          work, out_dev[lo:hi], nv, self.flags)
-                self.last_launches += 2  # lag kernel + finalize
+                self.last_launches += 2 if rg is None else 3  # lag kernel + finalize (+ per-block finalize)
         return out_dev
 
     def resolve_flags(self, table_dev, out_dev, nvalid_dev=None):
@@ -673,18 +711,28 @@ class LagSearchEngine:
             self.stats[:, 0].copy_(other.stats[:, 0])
         self.frame = other.frame
 
-    def search(self, table, planes=None, return_nvalid=False, lag_ij=None):
+    def search(self, table, planes=None, return_nvalid=False, lag_ij=None, block=None):
         """Host lag table [n_lags, k] -> numpy corr[n_lags]; shards over ranks when torch.distributed is up.
         lag_ij = (i1, i2[, group]): CRVAL1 / CRVAL2 grid indices of every lag (Carrington frame): each rank's slice is
-        handed to the kernel in `offset_patch_order`."""
+        handed to the kernel in `offset_patch_order`.
+        block = (rows, cols) (helioprojective frame, all-FP64 arithmetic): also the per-block cubes of the same pass;
+        returns (corr, nvalid, corr_blocks, nvalid_blocks), the last two [nby, nbx, n_lags] (blocks: `region_bounds`).
+        Each rank holds [chunk, n_blocks] of them; one all-gather assembles them."""
         torch = _torch()
         n = table.shape[0]
         dist, rank, world = _dist_info()
         chunk, bounds = shard_bounds(n, world)
         lo, hi = bounds[rank]
+        return_nvalid = return_nvalid or block is not None
         with torch.cuda.device(self.device):
             local = torch.full((chunk,), float("nan"), dtype=torch.float64, device=self.device)
             nvalid = torch.zeros(chunk, dtype=torch.int64, device=self.device) if return_nvalid else None
+            regions = None
+            if block is not None:
+                nby, nbx = _ext.region_grid(self.ref.shape[0], self.ref.shape[1], *block)
+                regions = (block[0], block[1],
+                           torch.full((nby * nbx, chunk), float("nan"), dtype=torch.float64, device=self.device),
+                           torch.zeros((nby * nbx, chunk), dtype=torch.int64, device=self.device))
             if hi > lo and lag_ij is not None and self.frame == "carrington":
                 out, nv = self.evaluate_patch_ordered(table[lo:hi], [np.asarray(v)[lo:hi] for v in lag_ij], planes,
                                                       return_nvalid=return_nvalid)
@@ -694,13 +742,19 @@ class LagSearchEngine:
             elif hi > lo:
                 tab_dev = self._upload(table[lo:hi])
                 nv = None if nvalid is None else nvalid[:hi - lo]
-                self.evaluate(tab_dev, local[:hi - lo], nv, planes)
+                self.evaluate(tab_dev, local[:hi - lo], nv, planes, regions=regions)
                 self.resolve_flags(tab_dev, local[:hi - lo], nv)
             full = gather_slices(local, n, chunk)
             corr = full.cpu().numpy()
             if return_nvalid:
                 nv_full = gather_slices(nvalid.to(torch.float64), n, chunk).cpu().numpy().astype(np.int64)
-                return corr, nv_full
+                if block is None:
+                    return corr, nv_full
+                # [chunk, 2, n_blocks] per rank: the block values of a lag travel with it
+                both = torch.stack([regions[2].t(), regions[3].t().to(torch.float64)], dim=1)
+                both = gather_slices(both, n, chunk).cpu().numpy()
+                return (corr, nv_full, both[:, 0].T.reshape(nby, nbx, n),
+                        both[:, 1].T.astype(np.int64).reshape(nby, nbx, n))
         return corr
 
 

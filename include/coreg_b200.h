@@ -262,6 +262,40 @@ int coreg_hpc_lag_corr_wcs(const float* ref_dev, const double* small_dev, int sn
                            int order, const double* pivots_dev, void* work_dev, size_t work_bytes, double* corr_dev,
                            int64_t* nvalid_dev, int flags, void* stream);
 
+/* ---- K1 with per-block outputs: local correlation cubes from the same pass --------------------------------------------
+ * The common grid is cut into blocks of block_h x block_w pixels starting at pixel (0, 0); the last block row and column
+ * take whatever remains: nby = ceil(gny / block_h), nbx = ceil(gnx / block_w), block (i, j) is row b = i * nbx + j of
+ * the outputs. Block sides are positive multiples of 64, so every block edge is a tile edge of both lag kernels and a
+ * block's moments are sums of the tile records the whole-grid fold reads.
+ *   corr_dev    [n_blocks][ld] float64 out: Pearson r of the block's pixels per lag (NaN where the block has no valid
+ *               pixel pair under that lag)
+ *   nvalid_dev  [n_blocks][ld] int64 out: the block's valid pixel pairs per lag; they sum to the whole-grid nvalid
+ *   ld          elements between consecutive blocks' rows, >= n_lags (a launch over a slice [lo, hi) of a longer lag
+ *               list writes columns lo .. hi - 1 when given corr_dev + lo, nvalid_dev + lo) */
+typedef struct CoregRegions {
+  int block_h, block_w;
+  int64_t ld;
+  double* corr_dev;
+  int64_t* nvalid_dev;
+} CoregRegions;
+
+/* coreg_hpc_lag_corr_wcs / coreg_hpc_lag_corr + a CoregRegions: the whole-grid outputs exactly as the call without it,
+ * then the per-block outputs, folded from the same tile records after the whole-grid finalize. A block's records are
+ * taken in ascending order and dealt to the accumulator groups as the whole-grid fold deals them, so one block covering
+ * the grid reproduces corr_dev / nvalid_dev bit for bit, and each lag's values depend only on its own records (not on
+ * how a lag list is split into launches or ranks). Returns COREG_EINVAL before any CUDA call when `regions` or one of
+ * its pointers is NULL, a block side is not a positive multiple of 64, ld < n_lags, the grid holds more than 65535
+ * blocks, or flags has COREG_FLAG_MIXED (the mixed kernel's per-lag guard is calibrated on whole-grid moments). */
+int coreg_hpc_lag_corr_wcs_regions(const float* ref_dev, const double* small_dev, int snx, int sny, int gnx, int gny,
+                                   const CoregTanWcs* grid_wcs_host, const CoregTanWcs* lag_wcs_dev, int64_t n_lags,
+                                   int order, const double* pivots_dev, void* work_dev, size_t work_bytes,
+                                   double* corr_dev, int64_t* nvalid_dev, const CoregRegions* regions, int flags,
+                                   void* stream);
+int coreg_hpc_lag_corr_regions(const float* ref_dev, const void* small_dev, int small_dtype, int snx, int sny, int gnx,
+                               int gny, const double* planes_dev, const CoregLagTan* lags_dev, int64_t n_lags, int order,
+                               const double* pivots_dev, void* work_dev, size_t work_bytes, double* corr_dev,
+                               int64_t* nvalid_dev, const CoregRegions* regions, int flags, void* stream);
+
 /* ---- K1 (fast form, mixed arithmetic; opt-in) ------------------------------------------------------------------------
  * coreg_hpc_lag_corr_wcs with the projection in FP64 and the spline + per-segment moments in FP32, for a small image
  * whose pixels are float32 values (a BITPIX -32 FITS payload: what `Fits.open(...)[w].data` holds before the
