@@ -86,8 +86,9 @@ def test_carrington_size_deg_grid_and_results_object(torch_cuda, toy_pair):
 def test_window_kernel_staging_paths_give_the_same_bits(torch_cuda, toy_pair, monkeypatch):
     """The Carrington kernel stages the reachable part of the small image in shared memory with one TMA tile load per
     (tile, lag chunk); COREG_NO_TMA=1 makes the block copy the window itself (what happens for images whose row pitch
-    is not a multiple of 16 bytes). Same arithmetic, same accumulation order: the cubes are bit-identical. A float64
-    small image (no float32 twin) goes through the float64 instantiation."""
+    is not a multiple of 16 bytes). Same arithmetic, same accumulation order: the cubes are bit-identical. The toy
+    pair's small image is float32; the float64 instantiation and the copy's own triggers (unaligned pitch or base)
+    are driven in test_gpu_carrington_window.py."""
     from euispice_coreg_b200.hdrshift import Alignment, engine
     lags = dict(LAGS, lag_crval1=np.arange(10, 38, 1.0), lag_crval2=np.arange(-6, 18, 1.0))
     grid = dict(lonlims=(246.0, 254.0), latlims=(-6.0, 2.0), shape=(150, 170))
