@@ -76,6 +76,8 @@ _SIGNATURES = {
                                     C.c_int, C.POINTER(CoregSurfaceFrames), _P, _P]),
     "coreg_hpc_lag_corr_edge": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int64, _P, _P,
                                           C.c_size_t, _P, _P, C.c_int, _P]),
+    "coreg_hpc_lag_corr_edge_regions": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int64, _P,
+                                                  _P, C.c_size_t, _P, _P, C.POINTER(CoregRegions), C.c_int, _P]),
     "coreg_surface_search_host": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.POINTER(CoregTanWcs), _P, C.c_int, C.c_int,
                                             C.c_int, C.POINTER(CoregTanWcs), C.POINTER(CoregSurfaceFrames), _P,
                                             C.c_int64, C.c_int, _P, _P]),
@@ -106,6 +108,9 @@ _SIGNATURES = {
     "coreg_carrington_planes": (C.c_int, [C.POINTER(CoregCarrington), _P, _P, C.c_int, _P, _P, C.c_int, _P, _P, _P]),
     "coreg_offset_lag_corr": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, C.c_int64,
                                         C.c_int, _P, _P, C.c_size_t, _P, _P, C.c_int, _P]),
+    "coreg_offset_lag_corr_regions": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P,
+                                                C.c_int64, C.c_int, _P, _P, C.c_size_t, _P, _P,
+                                                C.POINTER(CoregRegions), C.c_int, _P]),
     "coreg_car_pix2world": (C.c_int, [_P, C.c_int, C.c_int, _P, _P, _P]),
     "coreg_car_world2pix": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P]),
     "coreg_car_lag_corr": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, C.c_int64,
@@ -484,9 +489,10 @@ def surface_cut(wcs_small, wcs_large, large_pad, frames):
     return out
 
 
-def hpc_lag_corr_edge(ref, small_pad, planes, lags, pivots, work, corr_out, nvalid_out=None, flags=0):
+def hpc_lag_corr_edge(ref, small_pad, planes, lags, pivots, work, corr_out, nvalid_out=None, flags=0, regions=None):
     """Bilinear helioprojective search with reproject's edge rule (`coreg_hpc_lag_corr_edge`). `small_pad`: `pad_edge` of
-    the small image; `lags`: device float64 [n_lags, 12] (CoregLagTanEdge rows); `ref`: float64."""
+    the small image; `lags`: device float64 [n_lags, 12] (CoregLagTanEdge rows); `ref`: float64. `regions` =
+    (block_h, block_w, corr_blocks, nvalid_blocks): also the per-block outputs (`coreg_hpc_lag_corr_edge_regions`)."""
     torch = _torch()
     lib = load()
     _require_cuda(ref, small_pad, planes, lags, pivots, work, corr_out)
@@ -495,12 +501,16 @@ def hpc_lag_corr_edge(ref, small_pad, planes, lags, pivots, work, corr_out, nval
     if lags.shape[1] != LAG_TAN_EDGE_DOUBLES:
         raise TypeError("lags must be CoregLagTanEdge rows [n_lags, 12]")
     gny, gnx = ref.shape
+    args = (_ptr(ref), _ptr(small_pad), small_pad.shape[1] - 2, small_pad.shape[0] - 2, gnx, gny, _ptr(planes),
+            _ptr(lags), lags.shape[0], _ptr(pivots), _ptr(work), work.numel() * work.element_size(), _ptr(corr_out),
+            _ptr(nvalid_out) if nvalid_out is not None else None)
     with torch.cuda.device(ref.device):
-        _check(lib.coreg_hpc_lag_corr_edge(_ptr(ref), _ptr(small_pad), small_pad.shape[1] - 2, small_pad.shape[0] - 2,
-                                           gnx, gny, _ptr(planes), _ptr(lags), lags.shape[0], _ptr(pivots), _ptr(work),
-                                           work.numel() * work.element_size(), _ptr(corr_out),
-                                           _ptr(nvalid_out) if nvalid_out is not None else None, int(flags),
-                                           _stream()), "coreg_hpc_lag_corr_edge")
+        if regions is not None:
+            rg = _regions_struct(regions, gny, gnx, lags.shape[0])
+            _check(lib.coreg_hpc_lag_corr_edge_regions(*args, C.byref(rg), int(flags), _stream()),
+                   "coreg_hpc_lag_corr_edge_regions")
+            return
+        _check(lib.coreg_hpc_lag_corr_edge(*args, int(flags), _stream()), "coreg_hpc_lag_corr_edge")
 
 
 def hpc_lag_corr_wcs(ref, small, grid_wcs, lag_wcs, order, pivots, work, corr_out, nvalid_out=None, flags=0,
@@ -581,20 +591,25 @@ def carrington_planes(c: CoregCarrington, sinlon, coslon, sinlat, coslat):
     return tx, ty
 
 
-def offset_lag_corr(ref, small, tx, ty, lags, order, pivots, work, corr_out, nvalid_out=None, flags=0):
-    """K4. `lags`: device float64 [n_lags, 2] (CoregLagOffset rows)."""
+def offset_lag_corr(ref, small, tx, ty, lags, order, pivots, work, corr_out, nvalid_out=None, flags=0, regions=None):
+    """K4. `lags`: device float64 [n_lags, 2] (CoregLagOffset rows). `regions` = (block_h, block_w, corr_blocks,
+    nvalid_blocks): also the per-block outputs over the Carrington grid (`coreg_offset_lag_corr_regions`)."""
     torch = _torch()
     lib = load()
     _require_cuda(ref, small, tx, ty, lags, pivots, work, corr_out)
     if ref.dtype != torch.float64:
         raise TypeError("ref must be float64 (the reference keeps the Carrington-projected image in float64)")
     gny, gnx = ref.shape
+    args = (_ptr(ref), _ptr(small), _dt(small), small.shape[1], small.shape[0], gnx, gny, _ptr(tx), _ptr(ty),
+            _ptr(lags), lags.shape[0], int(order), _ptr(pivots), _ptr(work), work.numel() * work.element_size(),
+            _ptr(corr_out), _ptr(nvalid_out) if nvalid_out is not None else None)
     with torch.cuda.device(ref.device):
-        _check(lib.coreg_offset_lag_corr(_ptr(ref), _ptr(small), _dt(small), small.shape[1], small.shape[0], gnx, gny,
-                                         _ptr(tx), _ptr(ty), _ptr(lags), lags.shape[0], int(order), _ptr(pivots),
-                                         _ptr(work), work.numel() * work.element_size(), _ptr(corr_out),
-                                         _ptr(nvalid_out) if nvalid_out is not None else None,
-                                         int(flags), _stream()), "coreg_offset_lag_corr")
+        if regions is not None:
+            rg = _regions_struct(regions, gny, gnx, lags.shape[0])
+            _check(lib.coreg_offset_lag_corr_regions(*args, C.byref(rg), int(flags), _stream()),
+                   "coreg_offset_lag_corr_regions")
+            return
+        _check(lib.coreg_offset_lag_corr(*args, int(flags), _stream()), "coreg_offset_lag_corr")
 
 
 def _car_row(row):

@@ -519,5 +519,7 @@ int launch_finalize_tiles(const double* work, int tiles, int64_t n_lags, double*
 int launch_offset_fast(int gnx, int gny, int64_t n_lags, cudaStream_t s, const double* ref, const void* small,
                        int small_dtype, int snx, int sny, const double* tx, const double* ty,
                        const CoregLagOffset* lags, const double* pivots, void* work, double* corr, int64_t* nvalid);
+// per-block fold of the partials launch_offset_fast left in `work` (coreg_lag_offset.cu)
+int launch_offset_regions(int gnx, int gny, int64_t n_lags, const void* work, const CoregRegions* rg, cudaStream_t s);
 size_t offset_workspace_bytes(int gnx, int gny, int64_t n_lags);
 }  // namespace coreg

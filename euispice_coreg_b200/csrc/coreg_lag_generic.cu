@@ -219,6 +219,12 @@ int launch_lag(int gnx, int gny, int64_t n_lags, int sms, cudaStream_t s, const 
   return COREG_OK;
 }
 
+// the Carrington-frame window kernel serves the offset functor at order 2 with FMA arithmetic on images of at least
+// 3 x 3 pixels; every other offset search takes the generic kernel (which the per-block fold must follow)
+inline bool offset_window_applies(int order, int flags, int snx, int sny) {
+  return order == 2 && !(flags & COREG_FLAG_STRICT) && snx >= 3 && sny >= 3 && !(flags & COREG_FLAG_NO_FAST);
+}
+
 template <class Coord, typename SmallT, typename RefT, bool ROUND32>
 int launch_lag_corr(const RefT* ref, const SmallT* small, int snx, int sny, int gnx, int gny,
                     typename Coord::Planes planes, const typename Coord::Lag* lags, int64_t n_lags, int order,
@@ -233,8 +239,7 @@ int launch_lag_corr(const RefT* ref, const SmallT* small, int snx, int sny, int 
   const bool strict = (flags & COREG_FLAG_STRICT) != 0;
   double* w = static_cast<double*>(work);
   // window kernel for the offset (Carrington) functor: order 2, FMA arithmetic, image of at least 3x3
-  const bool fast_ok = std::is_same<Coord, OffsetCoord>::value && (order == 2) && !strict && snx >= 3 && sny >= 3 &&
-                       !(flags & COREG_FLAG_NO_FAST);
+  const bool fast_ok = std::is_same<Coord, OffsetCoord>::value && offset_window_applies(order, flags, snx, sny);
   if (work_bytes < (fast_ok ? offset_workspace_bytes(gnx, gny, n_lags) : coreg_lag_corr_workspace_bytes(gnx, gny, n_lags)))
     return fail(COREG_ENOMEM, "workspace too small");
   if constexpr (std::is_same<Coord, OffsetCoord>::value) {
@@ -354,6 +359,18 @@ int coreg_hpc_lag_corr_edge(const double* ref, const double* small_pad, int snx,
   return launch_finalize_tiles(static_cast<double*>(work), tiles, n_lags, corr, nvalid, s);
 }
 
+int coreg_hpc_lag_corr_edge_regions(const double* ref, const double* small_pad, int snx, int sny, int gnx, int gny,
+                                    const double* planes, const CoregLagTanEdge* lags, int64_t n_lags,
+                                    const double* pivots, void* work, size_t work_bytes, double* corr, int64_t* nvalid,
+                                    const CoregRegions* regions, int flags, void* stream) {
+  if (int rc = check_regions(regions, gnx, gny, n_lags, flags, "coreg_hpc_lag_corr_edge_regions")) return rc;
+  int rc = coreg_hpc_lag_corr_edge(ref, small_pad, snx, sny, gnx, gny, planes, lags, n_lags, pivots, work, work_bytes,
+                                   corr, nvalid, flags, stream);
+  if (rc || n_lags <= 0) return rc;
+  return launch_finalize_tiles_regions(static_cast<const double*>(work), gnx, gny, n_lags, regions,
+                                       (cudaStream_t)stream);
+}
+
 int coreg_offset_lag_corr(const double* ref, const void* small, int small_dtype, int snx, int sny, int gnx, int gny,
                           const double* tx, const double* ty, const CoregLagOffset* lags, int64_t n_lags, int order,
                           const double* pivots, void* work, size_t work_bytes, double* corr, int64_t* nvalid,
@@ -372,6 +389,21 @@ int coreg_offset_lag_corr(const double* ref, const void* small, int small_dtype,
                                                               n_lags, order, pivots, work, work_bytes, corr, nvalid,
                                                               flags, s);
   return fail(COREG_EINVAL, "small_dtype must be COREG_F32 or COREG_F64");
+}
+
+int coreg_offset_lag_corr_regions(const double* ref, const void* small, int small_dtype, int snx, int sny, int gnx,
+                                  int gny, const double* tx, const double* ty, const CoregLagOffset* lags,
+                                  int64_t n_lags, int order, const double* pivots, void* work, size_t work_bytes,
+                                  double* corr, int64_t* nvalid, const CoregRegions* regions, int flags, void* stream) {
+  if (int rc = check_regions(regions, gnx, gny, n_lags, flags, "coreg_offset_lag_corr_regions")) return rc;
+  int rc = coreg_offset_lag_corr(ref, small, small_dtype, snx, sny, gnx, gny, tx, ty, lags, n_lags, order, pivots,
+                                 work, work_bytes, corr, nvalid, flags, stream);
+  if (rc || n_lags <= 0) return rc;
+  // fold the records of the kernel that ran: the window kernel's slotted super-tile partials or the generic tiles
+  if (offset_window_applies(order, flags, snx, sny))
+    return launch_offset_regions(gnx, gny, n_lags, work, regions, (cudaStream_t)stream);
+  return launch_finalize_tiles_regions(static_cast<const double*>(work), gnx, gny, n_lags, regions,
+                                       (cudaStream_t)stream);
 }
 
 int coreg_car_lag_corr(const float* ref, const void* small, int small_dtype, int snx, int sny, int gnx, int gny,

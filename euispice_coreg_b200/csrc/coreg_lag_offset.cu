@@ -577,6 +577,49 @@ offset_finalize_kernel(const double* __restrict__ work, const int* __restrict__ 
   }
 }
 
+// Per-block form of offset_finalize_kernel (CoregRegions): blockIdx.y = block of the grid. The block's super-tiles are
+// walked in ascending index and their partials added serially from 0.0; slot order is ascending super-tile order, so
+// one block covering the grid adds the same partials in the same order as the whole-grid fold. A super-tile without a
+// slot in this launch contributes nothing, as in the whole-grid fold.
+__global__ void __launch_bounds__(256)
+offset_finalize_regions_kernel(const double* __restrict__ work, const int* __restrict__ slot_of_super, int n_lags,
+                               int sx_tiles, int sy_tiles, int bt_h, int bt_w, int nbx, double* __restrict__ corr,
+                               int64_t* __restrict__ nvalid, int64_t ld) {
+  __shared__ double s[32][kMom + 1];
+  const RegionTiles R = region_tiles(blockIdx.y, nbx, bt_h, bt_w, sx_tiles, sy_tiles);
+  const int l0 = blockIdx.x * 32, t = threadIdx.x, lag = l0 + t / kMom, q = t % kMom;
+  double acc = 0.0;
+  if (lag < n_lags) {
+    const double* p = work + (size_t)lag * kMom + q;
+    for (int k = 0; k < R.n_tiles; ++k) {
+      const int sl = slot_of_super[(R.ty0 + k / R.ntx) * sx_tiles + R.tx0 + k % R.ntx];
+      if (sl >= 0) acc += p[(size_t)sl * n_lags * kMom];
+    }
+  }
+  s[t / kMom][q] = acc;
+  __syncthreads();
+  if (t < 32 && l0 + t < n_lags) {
+    const size_t o = (size_t)blockIdx.y * ld + l0 + t;
+    corr[o] = pearson_from_moments(s[t][0], s[t][1], s[t][2], s[t][3], s[t][4], s[t][5]);
+    nvalid[o] = (int64_t)s[t][0];
+  }
+}
+
+// the per-block fold of the partials a launch_offset_fast call left in `work` (super-tiles of 32 x 64 grid pixels)
+int launch_offset_regions(int gnx, int gny, int64_t n_lags, const void* work, const CoregRegions* rg, cudaStream_t s) {
+  static_assert(kRegionAlign % kOffSuperH == 0 && kRegionAlign % kOffTileW == 0, "blocks hold whole super-tiles");
+  const OffWork L = offw_layout(gnx, gny, n_lags);
+  const char* base = static_cast<const char*>(work);
+  const int sx_tiles = (gnx + kOffTileW - 1) / kOffTileW, sy_tiles = (gny + kOffSuperH - 1) / kOffSuperH;
+  const int nbx = (gnx + rg->block_w - 1) / rg->block_w, nby = (gny + rg->block_h - 1) / rg->block_h;
+  offset_finalize_regions_kernel<<<dim3((unsigned)((n_lags + 31) / 32), (unsigned)(nbx * nby)), 256, 0, s>>>(
+      reinterpret_cast<const double*>(base + L.partials), reinterpret_cast<const int*>(base + L.slots), (int)n_lags,
+      sx_tiles, sy_tiles, rg->block_h / kOffSuperH, rg->block_w / kOffTileW, nbx, rg->corr_dev, rg->nvalid_dev,
+      rg->ld);
+  CK_LAUNCH("offset_finalize_regions_kernel");
+  return COREG_OK;
+}
+
 // ---- host side --------------------------------------------------------------------------------------------------
 typedef CUresult (*TensorMapEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                            const cuuint64_t*, const cuuint32_t*, const cuuint32_t*,

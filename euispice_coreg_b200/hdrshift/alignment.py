@@ -73,7 +73,8 @@ class Alignment:
             on the returned `AlignmentResults`. A shift that changes across the field (pointing drift along a SPICE
             raster, a roll or plate-scale error) shows up as block maxima that differ. Not with
             lag_search="coarse_to_fine" (its windows follow the global maximum), mixed arithmetic, or the Carrington
-            entry points.
+            entry points (`align_using_carrington` takes its blocks as an argument of the call, on the grid it
+            defines).
         """
         self.large_fov_known_pointing = large_fov_known_pointing
         self.small_fov_to_correct = small_fov_to_correct
@@ -162,12 +163,21 @@ class Alignment:
 
     def align_using_carrington(self, lonlims=None, latlims=None, size_deg_carrington=None, shape=None,
                                reference_date=None, method='correlation', method_carrington_reprojection="fa",
-                               return_type='AlignmentResults'):
+                               return_type='AlignmentResults', local_block=None):
         """Co-alignment on a user Carrington grid (`hdrshift/alignment.py:144-261`). method_carrington_reprojection:
         "fa" (`_carrington_transform_fa`, the default) or "sunpy" (`_carrington_transform_sunpy`, `:939-985`: no grid
         arguments needed; the search runs on the small image's own grid after a solar-surface reprojection of the large
-        image -- a restatement of sunpy / reproject's published algorithm, `_surface_search`)."""
+        image -- a restatement of sunpy / reproject's published algorithm, `_surface_search`).
+
+        local_block: None (default) or the block size (rows, cols) -- or one int for square blocks --, each a positive
+        multiple of 64, in pixels of the grid the search runs on: with "fa" the Carrington grid of this call (rows =
+        latitude samples, shape[1] of them; columns = longitude samples, shape[0] of them; both on the `linspace` grid
+        of lonlims / latlims), with "sunpy" the small image's own grid. The search then also returns one correlation
+        cube per block from the same pass of the lag kernel (`.local`, a `LocalAlignmentResults`, on this object and on
+        the returned `AlignmentResults`), e.g. latitude bands that see the longitude shift the rigid "fa" rotation
+        leaves. It applies to this call only; the constructor's `local_block` is refused here."""
         self._refuse_local_block("align_using_carrington")
+        block = None if local_block is None else _engine.local_block_shape(local_block)
         self.method = method
         self.coordinate_frame = "final_carrington"
         self.lon_ctype = "HPLN-TAN"
@@ -180,7 +190,7 @@ class Alignment:
         if method_carrington_reprojection == "sunpy":
             # (the reference reads no grid argument on this path: alignment.py:198-231 is the "fa" branch)
             self.lonlims = self.latlims = self.shape = self.reference_date = None
-            results = self._find_best_header_parameters()
+            results = self._find_best_header_parameters(carrington_block=block)
             return self._wrap_results(results, return_type)
         if reference_date is None:
             if "DATE-AVG" not in self.hdr_large:
@@ -203,7 +213,7 @@ class Alignment:
         if self.shape[0] * self.shape[1] > 25000000:
             warnings.warn(f"shape parameter is shape={shape}, which is very large."
                           "Computational time might significantly increase")
-        results = self._find_best_header_parameters()
+        results = self._find_best_header_parameters(carrington_block=block)
         return self._wrap_results(results, return_type)
 
     def align_using_initial_carrington(self, method='correlation', return_type='AlignmentResults'):
@@ -463,9 +473,11 @@ class Alignment:
     # ------------------------------------------------------------------------------------------------
     # the seam: lag grid -> correlation cube
     # ------------------------------------------------------------------------------------------------
-    def _find_best_header_parameters(self, ang2pipi: bool = True, fov_limits=None, remove_fov_limits=None):
+    def _find_best_header_parameters(self, ang2pipi: bool = True, fov_limits=None, remove_fov_limits=None,
+                                     carrington_block=None):
         """Correlation cube float64 [n_crval1, n_crval2, n_cdelt1, n_cdelt2, n_crota, n_solar_r]
-        (`alignment.py:613-797`, parallel branch)."""
+        (`alignment.py:613-797`, parallel branch). carrington_block: the (rows, cols) blocks of
+        `align_using_carrington(local_block=...)` (the helioprojective search reads `self.local_block`)."""
         if self.method != 'correlation':
             raise NotImplementedError("only method='correlation' is on the device path")
         self.local = self._local_raw = None
@@ -507,14 +519,7 @@ class Alignment:
             elif getattr(self, "local_block", None) is not None:
                 corr, nvalid, corr_b, nvalid_b = eng.search(table, block=self.local_block)
                 self.lags_evaluated = int(table.shape[0])
-                nb = corr_b.shape[:2]
-                if dead.any():       # dead lags read 0.0 in every block, as in the cube
-                    corr_b = np.where(dead, 0.0, corr_b)
-                cube_b = corr_b.reshape(nb + shape5 + (1,))
-                if n_r > 1:
-                    cube_b = np.repeat(cube_b, n_r, axis=-1)
-                bounds = _engine.region_bounds(eng.ref.shape[0], eng.ref.shape[1], self.local_block)
-                self._local_raw = (cube_b, nvalid_b.reshape(nb + shape5), bounds)
+                self._keep_local_blocks(eng.ref.shape, self.local_block, corr_b, nvalid_b, dead, shape5, n_r)
             else:
                 corr, nvalid = eng.search(table, return_nvalid=True)
                 self.lags_evaluated = int(table.shape[0])
@@ -543,15 +548,31 @@ class Alignment:
                 raise ValueError("lag_solar_r must hold exactly one value (the reference breaks on more, "
                                  "alignment.py:646-660)")
             if getattr(self, "method_carrington_reprojection", "fa") == "sunpy":
-                corr, nvalid = self._surface_search(eng, refs, d1, d2, d3, d4, d5, float(self.lag_solar_r[0]))
+                corr, nvalid, dead, blocks = self._surface_search(eng, refs, d1, d2, d3, d4, d5,
+                                                                  float(self.lag_solar_r[0]), carrington_block)
             else:
-                corr, nvalid = self._carrington_search(eng, refs, d1, d2, d3, d4, d5, float(self.lag_solar_r[0]))
+                corr, nvalid, dead, blocks = self._carrington_search(eng, refs, d1, d2, d3, d4, d5,
+                                                                     float(self.lag_solar_r[0]), carrington_block)
+            if blocks is not None:
+                self._keep_local_blocks(eng.ref.shape, carrington_block, *blocks, dead, shape5, n_r)
             cube[..., 0] = corr.reshape(shape5)
             self.nvalid = nvalid.reshape(shape5)
         else:
             raise NotImplementedError(self.coordinate_frame)
         self.data_large = None
         return cube
+
+    def _keep_local_blocks(self, grid_shape, block, corr_b, nvalid_b, dead, shape5, n_r):
+        """Per-block values [nby, nbx, n_lags] of a search over a (gny, gnx) grid -> `self._local_raw` (cube shape, lags
+        in `dead` 0.0 in every block as in the cube), wrapped into `self.local` with the results."""
+        nb = corr_b.shape[:2]
+        if dead is not None and dead.any():
+            corr_b = np.where(dead, 0.0, corr_b)
+        cube_b = corr_b.reshape(nb + shape5 + (1,))
+        if n_r > 1:
+            cube_b = np.repeat(cube_b, n_r, axis=-1)
+        bounds = _engine.region_bounds(grid_shape[0], grid_shape[1], block)
+        self._local_raw = (cube_b, nvalid_b.reshape(nb + shape5), bounds)
 
     def _coarse_to_fine(self, eng, table, shape5, w_large, dead=None):
         """Sub-lattice pass over the CRVAL1 x CRVAL2 plane, then dense windows around the running maximum (SURVEY.md
@@ -622,7 +643,7 @@ class Alignment:
         return _ext.CoregSurfaceFrames(g_lon, g_lat, g_d, i_lon, i_lat, i_d, (i_t - g_t) / 86400.0,
                                        d_solar_r * _engine.R_SUN_M)
 
-    def _surface_search(self, eng, refs, d1, d2, d3, d4, d5, d_solar_r):
+    def _surface_search(self, eng, refs, d1, d2, d3, d4, d5, d_solar_r, block=None):
         """`_carrington_transform_sunpy` (`alignment.py:939-985`) on the device. Once: the large image reprojected onto
         the small image's grid through sunpy's helioprojective -> helioprojective change of observer for points on the
         solar surface (radius d_solar_r R_sun), differentially rotated over the time between the two observations
@@ -630,19 +651,28 @@ class Alignment:
         lag: `Map(data_small, hdr_shifted).reproject_to(WCS(hdr_small))` -- same observer and time on both sides, so
         the change of frame is the identity and the call is the helioprojective search's geometry with bilinear
         interpolation and reproject's edge rule, no float32 store. sunpy / reproject are absent from the image: the
-        algorithm is restated from its published form (oracle/surface_reproject.py), parity unpinned."""
+        algorithm is restated from its published form (oracle/surface_reproject.py), parity unpinned.
+        Returns (corr, nvalid, dead, blocks): blocks = the per-block (corr, nvalid) [nby, nbx, n_lags] of the small
+        image's grid with `block`, else None."""
         w_small = TanWcs.from_header(self.hdr_small)
         w_large = TanWcs.from_header(self.hdr_large)
         eng.prepare_surface(self.data_large, w_large, w_small, self._surface_frames(d_solar_r))
         self.hdr_large = self.hdr_small.copy()
         table, dead = eng.surface_lag_table(self.hdr_small, refs, d1, d2, d3, d4, d5, self.cdelt_semantics)
-        corr, nvalid = eng.search(table, return_nvalid=True)
+        if block is None:
+            corr, nvalid = eng.search(table, return_nvalid=True)
+            blocks = None
+        else:
+            corr, nvalid, corr_b, nvalid_b = eng.search(table, block=block)
+            blocks = (corr_b, nvalid_b)
         self.lags_evaluated = int(table.shape[0])
-        return np.where(dead, 0.0, corr), nvalid
+        return np.where(dead, 0.0, corr), nvalid, dead, blocks
 
-    def _carrington_search(self, eng, refs, d1, d2, d3, d4, d5, d_solar_r):
+    def _carrington_search(self, eng, refs, d1, d2, d3, d4, d5, d_solar_r, block=None):
         """Per CROTA-lag value one pair of detector planes; CRVAL lags are pure offsets on them
-        (`alignment.py:889-901`, `utils/rectify.py:377-423`)."""
+        (`alignment.py:889-901`, `utils/rectify.py:377-423`). Returns (corr, nvalid, dead, blocks): blocks = the
+        per-block (corr, nvalid) [nby, nbx, n_lags] of the Carrington grid with `block` (every CROTA group's lags at
+        their place in the lag list; lags in `dead` are not evaluated and read 0.0 / 0), else None."""
         for hdr in (self.hdr_small, self.hdr_large):
             warn_fa_units(hdr)
         eng.prepare_carrington_large(self.data_large, self.hdr_large, d_solar_r, self.lonlims, self.latlims,
@@ -650,12 +680,20 @@ class Alignment:
         n = d1.size
         corr = np.zeros(n, dtype=np.float64)
         nvalid = np.zeros(n, dtype=np.int64)
+        blocks = None
+        if block is not None:
+            nb = _engine._ext.region_grid(eng.ref.shape[0], eng.ref.shape[1], *block)
+            blocks = (np.zeros(nb + (n,), dtype=np.float64), np.zeros(nb + (n,), dtype=np.int64))
         dead = carrington_dead_lags(d3, d4, self.cdelt_semantics)
         for sel, planes, table, lag_ij in self._carrington_tables(eng, refs, d1, d2, d5, dead, d_solar_r):
-            c, nv = eng.search(table, planes=planes, return_nvalid=True, lag_ij=lag_ij)
+            if block is None:
+                c, nv = eng.search(table, planes=planes, return_nvalid=True, lag_ij=lag_ij)
+            else:
+                c, nv, blocks[0][..., sel], blocks[1][..., sel] = eng.search(table, planes=planes, lag_ij=lag_ij,
+                                                                             block=block)
             corr[sel] = c
             nvalid[sel] = nv
-        return corr, nvalid
+        return corr, nvalid, dead, blocks
 
     def _carrington_tables(self, eng, refs, d1, d2, d5, dead, d_solar_r):
         """Per CROTA-lag value (generated one at a time: each holds a pair of planes the size of the grid):

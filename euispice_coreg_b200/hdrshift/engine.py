@@ -618,15 +618,17 @@ class LagSearchEngine:
         `tan_lag_table`) the generic one. Asynchronous. With mixed arithmetic `self.lag_flags` receives the per-lag
         guard verdicts: follow with `resolve_flags` (which synchronises) before trusting `out_dev`.
         regions = (rows, cols, corr_blocks [n_blocks, n] float64, nvalid_blocks [n_blocks, n] int64) device arrays
-        (helioprojective frame, all-FP64 arithmetic): also the per-block outputs of every lag, launch slice [lo, hi)
-        into columns [lo, hi)."""
+        (helioprojective frame with all-FP64 arithmetic, Carrington frame, "sunpy" surface frame): also the per-block
+        outputs of every lag, launch slice [lo, hi) into columns [lo, hi)."""
         torch = _torch()
         n = table_dev.shape[0]
         gny, gnx = self.ref.shape
         step = self.lags_per_launch(gnx, gny)
         self.last_launches = 0
-        if regions is not None and (self.frame != "hpc" or self.arithmetic == "mixed"):
-            raise ValueError("per-block outputs: helioprojective frame with all-FP64 arithmetic only")
+        if regions is not None and (self.frame not in ("hpc", "carrington", "surface") or
+                                    (self.frame == "hpc" and self.arithmetic == "mixed")):
+            raise ValueError("per-block outputs: helioprojective frame with all-FP64 arithmetic, Carrington and "
+                             "surface frames only")
         mixed = (allow_mixed and self.frame == "hpc" and table_dev.shape[1] == _ext.TAN_WCS_DOUBLES
                  and self._mixed_applies())
         with torch.cuda.device(self.device):
@@ -648,7 +650,7 @@ class LagSearchEngine:
                                           flagged=self.lag_flags[lo:hi] if mixed else None, regions=rg)
                 elif self.frame == "surface":
                     _ext.hpc_lag_corr_edge(self.ref, self.small_pad, self.planes, table_dev[lo:hi], self.pivots, work,
-                                           out_dev[lo:hi], nv, self.flags)
+                                           out_dev[lo:hi], nv, self.flags, regions=rg)
                 elif self.frame == "car":
                     _ext.car_lag_corr(self.ref, self.small, self.planes, table_dev[lo:hi], self.order,
                                       self.pivots, work, out_dev[lo:hi], nv, self.flags)
@@ -658,7 +660,7 @@ class LagSearchEngine:
                 else:
                     tx, ty = planes
                     _ext.offset_lag_corr(self.ref, self.small, tx, ty, table_dev[lo:hi], self.order, self.pivots,
-                                         work, out_dev[lo:hi], nv, self.flags)
+                                         work, out_dev[lo:hi], nv, self.flags, regions=rg)
                 self.last_launches += 2 if rg is None else 3  # lag kernel + finalize (+ per-block finalize)
         return out_dev
 
@@ -685,11 +687,14 @@ class LagSearchEngine:
             self.flagged_lags = k
         return k
 
-    def evaluate_patch_ordered(self, table, lag_ij, planes, return_nvalid=False, pinned=False):
+    def evaluate_patch_ordered(self, table, lag_ij, planes, return_nvalid=False, pinned=False, block=None):
         """Carrington frame, on this device alone: host offset table [n, 2] -> device corr [n] (and nvalid [n] or
         None), in the order of `table`. The lags are handed to the kernel in `offset_patch_order` of their grid indices
         lag_ij = (i1, i2[, group]) and scattered back. Asynchronous; pinned=True stages the uploads in page-locked
-        memory so that the host does not wait for the stream."""
+        memory so that the host does not wait for the stream.
+        block = (rows, cols): also the per-block values of the same pass, scattered back to table order like corr
+        (the dummy lags of the patch order dropped): returns (corr, nvalid, corr_blocks, nvalid_blocks), the last two
+        [n_blocks, n] (blocks: `region_bounds`)."""
         torch = _torch()
         slot, n_slots = offset_patch_order(*lag_ij)
         padded = np.full((n_slots, table.shape[1]), np.nan, dtype=np.float64)
@@ -699,8 +704,17 @@ class LagSearchEngine:
             idx = self._upload(slot, pinned=pinned)
             out = torch.empty(n_slots, dtype=torch.float64, device=self.device)
             nv = torch.empty(n_slots, dtype=torch.int64, device=self.device) if return_nvalid else None
-            self.evaluate(tab_dev, out, nv, planes)
-            return out.index_select(0, idx), (nv.index_select(0, idx) if return_nvalid else None)
+            regions = None
+            if block is not None:
+                n_blocks = int(np.prod(_ext.region_grid(self.ref.shape[0], self.ref.shape[1], *block)))
+                regions = (block[0], block[1],
+                           torch.empty((n_blocks, n_slots), dtype=torch.float64, device=self.device),
+                           torch.empty((n_blocks, n_slots), dtype=torch.int64, device=self.device))
+            self.evaluate(tab_dev, out, nv, planes, regions=regions)
+            res = out.index_select(0, idx), (nv.index_select(0, idx) if return_nvalid else None)
+            if block is None:
+                return res
+            return res + (regions[2].index_select(1, idx), regions[3].index_select(1, idx))
 
     def adopt_reference(self, other):
         """Search against `other`'s resident reference on the common grid (Carrington frame: one projection shared by
@@ -715,7 +729,7 @@ class LagSearchEngine:
         """Host lag table [n_lags, k] -> numpy corr[n_lags]; shards over ranks when torch.distributed is up.
         lag_ij = (i1, i2[, group]): CRVAL1 / CRVAL2 grid indices of every lag (Carrington frame): each rank's slice is
         handed to the kernel in `offset_patch_order`.
-        block = (rows, cols) (helioprojective frame, all-FP64 arithmetic): also the per-block cubes of the same pass;
+        block = (rows, cols) (frames as for `evaluate`'s regions): also the per-block cubes of the same pass;
         returns (corr, nvalid, corr_blocks, nvalid_blocks), the last two [nby, nbx, n_lags] (blocks: `region_bounds`).
         Each rank holds [chunk, n_blocks] of them; one all-gather assembles them."""
         torch = _torch()
@@ -734,11 +748,14 @@ class LagSearchEngine:
                            torch.full((nby * nbx, chunk), float("nan"), dtype=torch.float64, device=self.device),
                            torch.zeros((nby * nbx, chunk), dtype=torch.int64, device=self.device))
             if hi > lo and lag_ij is not None and self.frame == "carrington":
-                out, nv = self.evaluate_patch_ordered(table[lo:hi], [np.asarray(v)[lo:hi] for v in lag_ij], planes,
-                                                      return_nvalid=return_nvalid)
-                local[:hi - lo] = out
+                res = self.evaluate_patch_ordered(table[lo:hi], [np.asarray(v)[lo:hi] for v in lag_ij], planes,
+                                                  return_nvalid=return_nvalid, block=block)
+                local[:hi - lo] = res[0]
                 if return_nvalid:
-                    nvalid[:hi - lo] = nv
+                    nvalid[:hi - lo] = res[1]
+                if block is not None:
+                    regions[2][:, :hi - lo] = res[2]
+                    regions[3][:, :hi - lo] = res[3]
             elif hi > lo:
                 tab_dev = self._upload(table[lo:hi])
                 nv = None if nvalid is None else nvalid[:hi - lo]

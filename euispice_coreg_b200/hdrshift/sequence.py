@@ -86,14 +86,52 @@ def _refs(a):
     return refs
 
 
+def gather_frame_blocks(blocks, n_frames, n_lags, device):
+    """{frame index: ((gny, gnx), corr [n_blocks, n_lags], nvalid [n_blocks, n_lags])} of this rank's frames (per-block
+    values of `align_using_carrington(local_block=...)`) -> the same for ALL frames, on every rank: one more all-gather
+    of `gather_frame_cubes`' [frames per rank, width] shape. A row carries gny, gnx, n_blocks, corr and nvalid as
+    float64 (the counts are exact below 2^53); its width, that of the frame with the most blocks, is agreed on by a
+    one-element max all-reduce, because a rank without frames does not know it and the "sunpy" grid is each frame's
+    own."""
+    torch = _engine._torch()
+    dist, rank, world = _engine._dist_info()
+    if dist is None or world == 1 or n_frames == 0:
+        return blocks
+    rows = {k: np.concatenate([[grid[0], grid[1], c.shape[0]], c.ravel(), nv.ravel().astype(np.float64)])
+            for k, (grid, c, nv) in blocks.items()}
+    width = torch.tensor([max([r.size for r in rows.values()] + [3])], dtype=torch.int64, device=device)
+    dist.all_reduce(width, op=dist.ReduceOp.MAX)
+    width = int(width.item())
+    rows = {k: np.pad(r, (0, width - r.size), constant_values=np.nan) for k, r in rows.items()}
+    out = {}
+    for k, r in gather_frame_cubes(rows, n_frames, width, device).items():
+        nb = int(r[2])
+        m = nb * n_lags
+        out[k] = ((int(r[0]), int(r[1])), r[3:3 + m].reshape(nb, n_lags), r[3 + m:3 + 2 * m].astype(np.int64)
+                  .reshape(nb, n_lags))
+    return out
+
+
+def _block_buffers(e, block, n_lags):
+    """This frame's per-block outputs on engine `e`'s grid: ((gny, gnx), corr, nvalid), [n_blocks, n_lags] zeros on the
+    device (lags never evaluated read 0.0 / 0, as in the cube); None without `block`."""
+    if block is None:
+        return None
+    torch = _engine._torch()
+    n_blocks = int(np.prod(_engine._ext.region_grid(e.ref.shape[0], e.ref.shape[1], *block)))
+    return (tuple(e.ref.shape), torch.zeros((n_blocks, n_lags), dtype=torch.float64, device=e.device),
+            torch.zeros((n_blocks, n_lags), dtype=torch.int64, device=e.device))
+
+
 class _Frame:
     """One frame in flight: its host-side `Alignment`, the mask of lags that read 0.0, the device result [n_lags], the
-    call that enqueues its search on the current stream and, optionally, the call that completes the result on the
-    side stream before it is fetched."""
-    __slots__ = ("a", "dead", "out", "search", "resolve")
+    call that enqueues its search on the current stream, optionally the call that completes the result on the side
+    stream before it is fetched, and optionally its per-block outputs ((gny, gnx), corr [n_blocks, n_lags],
+    nvalid [n_blocks, n_lags]) on the device."""
+    __slots__ = ("a", "dead", "out", "search", "resolve", "blocks")
 
-    def __init__(self, a, dead, out, search, resolve=None):
-        self.a, self.dead, self.out, self.search, self.resolve = a, dead, out, search, resolve
+    def __init__(self, a, dead, out, search, resolve=None, blocks=None):
+        self.a, self.dead, self.out, self.search, self.resolve, self.blocks = a, dead, out, search, resolve, blocks
 
 
 class SequenceAlignment:
@@ -217,7 +255,7 @@ class SequenceAlignment:
 
     def align_using_carrington(self, lonlims=None, latlims=None, shape=None, reference_date=None,
                                method_carrington_reprojection="fa", return_type="AlignmentResults",
-                               size_deg_carrington=None):
+                               size_deg_carrington=None, local_block=None):
         """Carrington-frame search of every frame against the reference: the cube of each frame is the one of
         `Alignment(reference, frame, ...).align_using_carrington(...)` with the same arguments. -> list (one entry per
         frame, input order) of `AlignmentResults` or, with return_type="corr", of cubes float64
@@ -227,8 +265,15 @@ class SequenceAlignment:
         planes of each distinct CROTA lag and the offset-window search. Only an explicit lonlims / latlims / shape grid
         is accepted (size_deg_carrington would centre a different grid on every frame). "sunpy": the reference is
         uploaded and edge-padded once; per frame, its solar-surface cut onto the frame's grid and the bilinear search
-        (grid arguments are not read, as in `Alignment`)."""
+        (grid arguments are not read, as in `Alignment`).
+
+        local_block: as in `Alignment.align_using_carrington`; each frame's `AlignmentResults` then carries `.local`,
+        the per-block cubes of that frame's search. Not with return_type="corr", which returns the cubes alone."""
         torch = _engine._torch()
+        block = None if local_block is None else _engine.local_block_shape(local_block)
+        if block is not None and return_type == "corr":
+            raise ValueError('local_block needs return_type="AlignmentResults" (the per-block cubes travel on the '
+                             "results objects)")
         hdr_large, data_large, reference_date, d_solar_r = self._check_carrington(
             lonlims, latlims, shape, reference_date, method_carrington_reprojection, size_deg_carrington)
         engs = self._engines(small_storage="auto")
@@ -245,7 +290,9 @@ class SequenceAlignment:
                 table, dead = e.surface_lag_table(a.hdr_small, _refs(a), *_lag_grid(a), a.cdelt_semantics)
                 tab_dev = e._upload(table, pinned=True)
                 out = torch.empty(table.shape[0], dtype=torch.float64, device=e.device)
-                return _Frame(a, dead, out, lambda: e.evaluate(tab_dev, out))
+                blocks = _block_buffers(e, block, table.shape[0])
+                regions = None if blocks is None else block + blocks[1:]
+                return _Frame(a, dead, out, lambda: e.evaluate(tab_dev, out, regions=regions), blocks=blocks)
         else:
             engs[0].prepare_carrington_large(data_large, hdr_large, d_solar_r, lonlims, latlims, shape)
             engs[1].adopt_reference(engs[0])
@@ -262,22 +309,27 @@ class SequenceAlignment:
                           for sel, planes, table, lag_ij in a._carrington_tables(e, _refs(a), d1, d2, d5, dead,
                                                                                  d_solar_r)]
                 out = torch.zeros(d1.size, dtype=torch.float64, device=e.device)
+                blocks = _block_buffers(e, block, d1.size)
 
                 def search():
                     for sel_dev, planes, table, lag_ij in groups:
-                        corr, _ = e.evaluate_patch_ordered(table, lag_ij, planes, pinned=True)
-                        out.index_copy_(0, sel_dev, corr)
-                return _Frame(a, dead, out, search)
+                        res = e.evaluate_patch_ordered(table, lag_ij, planes, pinned=True, block=block)
+                        out.index_copy_(0, sel_dev, res[0])
+                        if blocks is not None:
+                            blocks[1].index_copy_(1, sel_dev, res[2])
+                            blocks[2].index_copy_(1, sel_dev, res[3])
+                return _Frame(a, dead, out, search, blocks=blocks)
 
-        return self._run(engs, prepare, return_type, "final_carrington")
+        return self._run(engs, prepare, return_type, "final_carrington", block)
 
-    def _run(self, engs, prepare, return_type, coordinate_frame):
+    def _run(self, engs, prepare, return_type, coordinate_frame, block=None):
         """The frame loop of every search frame. `prepare(path, engine)` runs with the side stream current once that
         engine's previous search has finished: host reading and preparation of the frame (overlapping the device
         search of the previous frame), its uploads and its one-time device steps; it returns a `_Frame`, whose search
         is then enqueued on the main stream. The cube of frame k is fetched after frame k+1 has been enqueued. With
         torch.distributed up, this rank searches its own frames (`frames_of_rank`) and the cubes are all-gathered:
-        every rank returns all frames."""
+        every rank returns all frames. block: the (rows, cols) of frames that carry per-block outputs, fetched and
+        gathered with the cubes and attached to the results as `.local`."""
         import time
         torch = _engine._torch()
         dist, rank, world = _engine._dist_info()
@@ -294,6 +346,7 @@ class SequenceAlignment:
             shape5 = _shape5(self._host_prepare(self.list_small[0], coordinate_frame))
         pending = None                                      # (frame index, _Frame, event after its search, engine)
         cubes = {}
+        blocks = {}
         aligns = {}
 
         def finish(item):
@@ -306,6 +359,9 @@ class SequenceAlignment:
                 if fr.resolve is not None:
                     fr.resolve()
                 host = fr.out.cpu()
+                if fr.blocks is not None:
+                    grid, corr_b, nvalid_b = fr.blocks
+                    blocks[k] = (grid, np.where(fr.dead, 0.0, corr_b.cpu().numpy()), nvalid_b.cpu().numpy())
                 if e.small_count() == 0:     # (this engine's statistics still describe frame k: see above)
                     raise ValueError("minimum or maximum value have set all small FOV to nan")
             cubes[k] = np.where(fr.dead, 0.0, host.numpy())
@@ -341,6 +397,8 @@ class SequenceAlignment:
         # assemble: every rank ends with all cubes (one all-gather of [frames per rank, n_lags])
         n_lags = int(np.prod(shape5)) if shape5 is not None else 0
         cubes = gather_frame_cubes(cubes, n_frames, n_lags, eng.device)
+        if block is not None:
+            blocks = gather_frame_blocks(blocks, n_frames, n_lags, eng.device)
         out = []
         for k in range(n_frames):
             cube = cubes[k].reshape(shape5 + (1,))
@@ -353,5 +411,10 @@ class SequenceAlignment:
             if a is None:                                   # frame searched by another rank: host prep only
                 a = self._host_prepare(self.list_small[k], coordinate_frame)
                 a.data_small = None
+            if block is not None:
+                grid, corr_b, nvalid_b = blocks[k]
+                nb = _engine._ext.region_grid(grid[0], grid[1], *block)
+                a._keep_local_blocks(grid, block, corr_b.reshape(nb + (-1,)), nvalid_b.reshape(nb + (-1,)), None,
+                                     shape5, n_r)
             out.append(a._wrap_results(cube, "AlignmentResults"))
         return out

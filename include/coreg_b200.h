@@ -358,6 +358,28 @@ int coreg_offset_lag_corr(const double* ref_dev, const void* small_dev, int smal
                           int64_t n_lags, int order, const double* pivots_dev, void* work_dev, size_t work_bytes,
                           double* corr_dev, int64_t* nvalid_dev, int flags, void* stream);
 
+/* ---- Carrington-frame searches with per-block outputs (CoregRegions, as for K1 above) ----------------------------------
+ * coreg_offset_lag_corr_regions: coreg_offset_lag_corr + a CoregRegions over the Carrington grid (rows = latitude
+ *   samples, columns = longitude samples). The whole-grid outputs are exactly those of the call without it; then the
+ *   per-block fold of the records of the kernel that ran: the window kernel's partials (one per live 32 x 64-pixel
+ *   super-tile and lag, a block's super-tiles added in ascending order from 0.0, as the whole-grid fold adds its slots),
+ *   or, for orders 0, 1, 3, COREG_FLAG_STRICT, COREG_FLAG_NO_FAST and images smaller than 3 x 3, the generic kernel's
+ *   tile partials. A super-tile that no lag of a launch can bring onto the small image holds no partial and adds
+ *   nothing, so a lag's block values do not depend on the launch it was part of.
+ * coreg_hpc_lag_corr_edge_regions: coreg_hpc_lag_corr_edge + a CoregRegions over the small image's grid (the "sunpy"
+ *   search), folded from the generic kernel's tile partials.
+ * Both: one block covering the grid reproduces corr_dev / nvalid_dev bit for bit; COREG_EINVAL before any CUDA call on
+ * the conditions of coreg_hpc_lag_corr_regions. */
+int coreg_offset_lag_corr_regions(const double* ref_dev, const void* small_dev, int small_dtype, int snx, int sny,
+                                  int gnx, int gny, const double* tx_dev, const double* ty_dev,
+                                  const CoregLagOffset* lags_dev, int64_t n_lags, int order, const double* pivots_dev,
+                                  void* work_dev, size_t work_bytes, double* corr_dev, int64_t* nvalid_dev,
+                                  const CoregRegions* regions, int flags, void* stream);
+int coreg_hpc_lag_corr_edge_regions(const double* ref_dev, const double* small_pad_dev, int snx, int sny, int gnx,
+                                    int gny, const double* planes_dev, const CoregLagTanEdge* lags_dev, int64_t n_lags,
+                                    const double* pivots_dev, void* work_dev, size_t work_bytes, double* corr_dev,
+                                    int64_t* nvalid_dev, const CoregRegions* regions, int flags, void* stream);
+
 /* ---- plate-carree (-CAR) images: the frame of Alignment.align_using_initial_carrington ------------------------------
  * hdrshift/alignment.py:344-399: both images already are Carrington maps; the search is the helioprojective one with
  * the CAR projection in place of TAN and no longitude wrapping (utils/Util.py:295-305).
