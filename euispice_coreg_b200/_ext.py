@@ -136,6 +136,7 @@ _SIGNATURES = {
                                                C.c_int, _P, _P]),
     "coreg_synras_build_host": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(CoregTanWcs),
                                           C.POINTER(C.c_int), _P, _P, C.c_int, C.c_int, C.c_int, _P]),
+    "coreg_gauss2d_fit": (C.c_int, [_P, _P, _P, _P, C.c_int64, _P, _P, _P, _P, _P]),
     "coreg_fp64_peak": (C.c_int, [C.POINTER(C.c_double), C.c_int, _P]),
     "coreg_profile_begin": (C.c_int, []),
     "coreg_profile_end": (C.c_int, [C.POINTER(C.c_double), C.POINTER(C.c_int)]),
@@ -854,6 +855,33 @@ def synras_build_host(frames, wcs_list, frame_of_col, lng, lat, order):
                                        lng.ctypes.data_as(_P), lat.ctypes.data_as(_P), n_rows, n_cols, int(order),
                                        out.ctypes.data_as(_P)), "coreg_synras_build_host")
     return out
+
+
+FIT_MAX_POINTS = 26     # COREG_FIT_MAX_POINTS: points of one Gaussian peak fit
+FIT_CONVERGED, FIT_NOT_CONVERGED = 0, 3
+
+
+def gauss2d_fit(points, n_points, p0, bounds):
+    """Batched bounded 2-D Gaussian fits (`coreg_gauss2d_fit`). points: device float64 [n, 26, 3] (x, y, value);
+    n_points: int32 [n]; p0: float64 [n, 6]; bounds: float64 [n, 12] (lo then hi). Returns device (popt [n, 6],
+    cost [n], iterations [n] int32, status [n] int32: FIT_CONVERGED or FIT_NOT_CONVERGED). Asynchronous."""
+    torch = _torch()
+    lib = load()
+    _require_cuda(points, n_points, p0, bounds)
+    n = points.shape[0]
+    if points.dtype != torch.float64 or p0.dtype != torch.float64 or bounds.dtype != torch.float64 or \
+            n_points.dtype != torch.int32:
+        raise TypeError("gauss2d_fit: float64 points / p0 / bounds and int32 n_points")
+    if points.shape != (n, FIT_MAX_POINTS, 3) or n_points.shape != (n,) or p0.shape != (n, 6) or bounds.shape != (n, 12):
+        raise ValueError("gauss2d_fit: points [n, 26, 3], n_points [n], p0 [n, 6], bounds [n, 12]")
+    popt = torch.empty((n, 6), dtype=torch.float64, device=points.device)
+    cost = torch.empty(n, dtype=torch.float64, device=points.device)
+    iters = torch.empty(n, dtype=torch.int32, device=points.device)
+    status = torch.empty(n, dtype=torch.int32, device=points.device)
+    with torch.cuda.device(points.device):
+        _check(lib.coreg_gauss2d_fit(_ptr(points), _ptr(n_points), _ptr(p0), _ptr(bounds), n, _ptr(popt), _ptr(cost),
+                                     _ptr(iters), _ptr(status), _stream()), "coreg_gauss2d_fit")
+    return popt, cost, iters, status
 
 
 def fp64_peak(iters=20000):

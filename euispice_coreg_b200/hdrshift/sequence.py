@@ -20,6 +20,7 @@ edge-padded once; per frame its solar-surface cut onto the frame's grid is new. 
 """
 from __future__ import annotations
 
+import os
 import warnings
 
 import numpy as np
@@ -192,10 +193,20 @@ class SequenceAlignment:
                                         arithmetic=self.kw["arithmetic"], small_storage=small_storage)
                 for _ in range(2)]
 
-    def align_using_helioprojective(self, return_type="AlignmentResults"):
+    def align_using_helioprojective(self, return_type="AlignmentResults", local_block=None):
         """-> list (one entry per frame, input order) of `AlignmentResults` or, with return_type="corr", of cubes
-        float64 [n_crval1, n_crval2, n_cdelt1, n_cdelt2, n_crota, 1]."""
+        float64 [n_crval1, n_crval2, n_cdelt1, n_cdelt2, n_crota, 1].
+
+        local_block: None (default) or the block size (rows, cols) -- or one int for square blocks --, each a positive
+        multiple of 64, in pixels of each frame's common grid: each frame's `AlignmentResults` then carries `.local`,
+        the per-block cubes of that frame's search, equal to those of `Alignment(reference, frame, ...,
+        local_block=...).align_using_helioprojective()`. Not with return_type="corr", which returns the cubes alone, and
+        not with mixed arithmetic."""
         torch = _engine._torch()
+        block = self._local_block_of_call(local_block, return_type)
+        if block is not None and (self.kw["arithmetic"] or os.environ.get("COREG_ARITHMETIC")) == "mixed":
+            raise ValueError("local_block needs all-FP64 arithmetic (the mixed kernel's per-lag guard is calibrated on "
+                             "whole-grid moments)")
         engs = self._engines()
         # the reference image: read, checked and uploaded once
         hdr_large, data_large = self._open_reference()
@@ -209,10 +220,21 @@ class SequenceAlignment:
             table, dead = e.hpc_lag_table(a.hdr_small, _refs(a), *_lag_grid(a), a.cdelt_semantics)
             tab_dev = e._upload(table, pinned=True)
             out = torch.empty(table.shape[0], dtype=torch.float64, device=e.device)
+            blocks = _block_buffers(e, block, table.shape[0])
+            regions = None if blocks is None else block + blocks[1:]
             # mixed arithmetic (opt-in): lags that tripped the kernel's guard are redone in FP64 on the side stream
-            return _Frame(a, dead, out, lambda: e.evaluate(tab_dev, out), lambda: e.resolve_flags(tab_dev, out))
+            return _Frame(a, dead, out, lambda: e.evaluate(tab_dev, out, regions=regions),
+                          lambda: e.resolve_flags(tab_dev, out), blocks)
 
-        return self._run(engs, prepare, return_type, "final_helioprojective")
+        return self._run(engs, prepare, return_type, "final_helioprojective", block)
+
+    @staticmethod
+    def _local_block_of_call(local_block, return_type):
+        block = None if local_block is None else _engine.local_block_shape(local_block)
+        if block is not None and return_type == "corr":
+            raise ValueError('local_block needs return_type="AlignmentResults" (the per-block cubes travel on the '
+                             "results objects)")
+        return block
 
     def _check_carrington(self, lonlims, latlims, shape, reference_date, method_carrington_reprojection,
                           size_deg_carrington):
@@ -270,10 +292,7 @@ class SequenceAlignment:
         local_block: as in `Alignment.align_using_carrington`; each frame's `AlignmentResults` then carries `.local`,
         the per-block cubes of that frame's search. Not with return_type="corr", which returns the cubes alone."""
         torch = _engine._torch()
-        block = None if local_block is None else _engine.local_block_shape(local_block)
-        if block is not None and return_type == "corr":
-            raise ValueError('local_block needs return_type="AlignmentResults" (the per-block cubes travel on the '
-                             "results objects)")
+        block = self._local_block_of_call(local_block, return_type)
         hdr_large, data_large, reference_date, d_solar_r = self._check_carrington(
             lonlims, latlims, shape, reference_date, method_carrington_reprojection, size_deg_carrington)
         engs = self._engines(small_storage="auto")

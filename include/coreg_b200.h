@@ -511,6 +511,26 @@ int coreg_synras_build_host(const void* frames_host, int frame_dtype, int n_fram
                             const CoregTanWcs* wcs_host, const int* frame_of_col_host, const double* lng_host,
                             const double* lat_host, int n_rows, int n_cols, int order, double* out_host);
 
+/* ---- batched bounded 2-D Gaussian peak fits ---------------------------------------------------------------------------
+ * The sub-lag fit of AlignmentResults._compute_shift (scipy curve_fit of twoD_Gaussian, bounded, on the points around a
+ * cube's maximum) for n_problems cubes at once: least squares of
+ *   f(x, y) = p5 + p0 exp(-((x - p1)^2 / (2 p3^2) + (y - p2)^2 / (2 p4^2)))
+ * within lo <= p <= hi, by a bounded Levenberg-Marquardt with an active set, FP64, one warp per problem; sigma (p3, p4)
+ * stays strictly above its lower bound. Deterministic: a problem's result does not depend on the batch it is in.
+ *   points_dev     [n_problems][COREG_FIT_MAX_POINTS][3] float64: (x, y, value) of each point, the first n_points used
+ *   n_points_dev   [n_problems] int32, 1 .. COREG_FIT_MAX_POINTS (other counts give COREG_FIT_NOT_CONVERGED)
+ *   p0_dev         [n_problems][6] start, inside the bounds; bounds_dev [n_problems][12]: lo[6] then hi[6]
+ *   popt_dev       [n_problems][6] out; cost_dev [n_problems] out: sum of squared residuals at popt
+ *   iterations_dev [n_problems] int32 out; status_dev [n_problems] int32 out: COREG_FIT_CONVERGED or
+ *                  COREG_FIT_NOT_CONVERGED (iteration cap reached, or a non-finite cost at the start)
+ * Asynchronous on `stream`. COREG_EINVAL before any CUDA call for a null pointer or n_problems < 0. */
+#define COREG_FIT_MAX_POINTS 26
+#define COREG_FIT_CONVERGED 0
+#define COREG_FIT_NOT_CONVERGED 3
+int coreg_gauss2d_fit(const double* points_dev, const int* n_points_dev, const double* p0_dev, const double* bounds_dev,
+                      int64_t n_problems, double* popt_dev, double* cost_dev, int* iterations_dev, int* status_dev,
+                      void* stream);
+
 /* Measurement hooks (bench.py): between begin and end every fused lag-kernel launch made by the calling thread is
  * bracketed by a CUDA event pair on its own stream; end() synchronises on them and returns the summed device time
  * of those launches [ms] and their count. No effect on results. */
